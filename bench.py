@@ -2,7 +2,7 @@
 """Benchmark of the OffsetGuided post-network decoder on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
-                    [--workload cfg2|cfg3|cfg4] [--batch B] [--long-edge E]
+                    [--workload cfg2|cfg3|cfg4] [--batch B] [--long-edge E] [--dump-outputs DIR]
 
 One "step" decodes ONE GLOBAL BATCH of synthetic network outputs, sharded by image over the N
 ranks (strong scaling: ceil(B / N) images per GPU, no collective on the data path).  Default
@@ -26,6 +26,10 @@ to 640x640, topk 32, thre-hmp 0.04, person-thre 0.04, dist-max 40) at the north-
   cpu_baseline     the oracle port of the reference decoder on the host cores (N = 1 only).
 
 `--impl reference` times the CPU oracle port alone on the same global batch (rank 0 only).
+
+`--dump-outputs DIR` writes, after the timed steps, the poses the timed path returned for its last
+step: one (M_i, C, 6) float32 array per image as DIR/poses_<global image index>.npy.  The inputs are
+seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -46,6 +50,7 @@ METRIC = 'decoded images/s @640 long-edge'
 UNIT = 'images/s'
 MIN_LEN = 0.5
 L2_BYTES = 126e6
+DUMP_BYTES = 64 << 20
 
 
 def parse_args():
@@ -62,7 +67,12 @@ def parse_args():
     ap.add_argument('--hot-only', action='store_true',
                     help='run only the HBM-resident full-resolution hot path (for ncu captures; no bench line)')
     ap.add_argument('--lean', action='store_true', help='skip the extra legs (weak scaling, sustained run, baselines)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the poses of the last timed step as DIR/poses_<image>.npy (float32)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    return args
 
 
 def workload(args):
@@ -106,6 +116,21 @@ def workload_config(w, n_gpus, per_gpu):
                                                      w['batch'] * w['c'] * e * e * 4 / 1e9),
         'persons_per_image': w['persons'],
     }
+
+
+def dump_outputs(out_dir, poses, first, n_images, w):
+    """Write `poses` (the per-image results of images first, first + 1, ... of a batch of `n_images`)
+    as out_dir/poses_<image>.npy.  An image has at most L * K persons; when that bound allows more
+    than DUMP_BYTES in all, a fixed seeded sample of the images is written, chosen from the arguments
+    alone so that every build writes the same files."""
+    images = np.arange(n_images)
+    cap = DUMP_BYTES // (w['l'] * w['topk'] * w['c'] * 6 * 4)
+    if n_images > cap:
+        images = np.sort(np.random.RandomState(0).permutation(n_images)[:cap])
+    os.makedirs(out_dir, exist_ok=True)
+    for g in images:
+        if first <= g < first + len(poses):
+            np.save(os.path.join(out_dir, 'poses_%05d.npy' % g), np.asarray(poses[g - first], dtype=np.float32))
 
 
 # --------------------------------------------------------------------------- inputs
@@ -260,7 +285,7 @@ def run_reference(args):
         run(hmp, omp, flip)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        run(hmp, omp, flip)
+        poses = run(hmp, omp, flip)
     dt = time.perf_counter() - t0
     value = n_images * args.steps / dt
     sample = '%d images per step (the global batch is %d), %d steps after %d warm-up steps, %s' % (
@@ -274,6 +299,8 @@ def run_reference(args):
         'e2e': {'value': value, 'unit': UNIT, 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0},
         'gpu_launches': 0,
     }))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, poses, 0, n_images, w)
 
 
 # --------------------------------------------------------------------------- B200 arm
@@ -474,7 +501,7 @@ def run_b200(args):
     v0, v1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.perf_counter()
     v0.record()
-    pipelined(post, feats_ring, flip, args.steps, depth)
+    last_poses = pipelined(post, feats_ring, flip, args.steps, depth)
     v1.record()
     torch.cuda.synchronize(dev)
     value_wall_ms = (time.perf_counter() - t0) * 1e3
@@ -714,6 +741,8 @@ def run_b200(args):
             'clocks': clocks,
         }
         print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_poses, start_i, B, w)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
