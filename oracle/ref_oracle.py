@@ -269,11 +269,16 @@ def person_score(row, index):
 
 
 def group_skeletons(limbs, skeleton, n_keypoints, person_thre, sort_dim=2,
-                    dist_max=10, use_scale=False, stats=None):
+                    dist_max=10, use_scale=False, stats=None, trace=None):
     """decoder/group.py:39-185 for ONE image, written as explicit sequential
     loops so that every numpy fancy-indexing subtlety of the reference is spelled
     out (last write wins, right-hand sides read the pre-update state, mask_sum
     resets only when at least one pair passed, column-sum cancellation).
+
+    ``trace`` (a list) receives one tuple (li, mm, kk, n_new, n_merged) per limb
+    step that has kept rows: persons at the start of the step, kept rows, persons
+    the step starts and persons it merges away.  The sum of n_new is the number of
+    person rows a table that never recycles rows needs.
 
     limbs: (L, K, 13) float32.  Returns (M, C, 6) float32
     [x, y, v, s, limb_score, ind]."""
@@ -345,6 +350,7 @@ def group_skeletons(limbs, skeleton, n_keypoints, person_thre, sort_dim=2,
                         msum[m][k] = -1
 
         # -- merge persons that now share exactly two keypoints (:140-161)
+        n_merged = 0
         if mm >= 2:
             ids = [[int(v) for v in r[:, 5]] for r in subset]
             mpairs = []
@@ -362,8 +368,10 @@ def group_skeletons(limbs, skeleton, n_keypoints, person_thre, sort_dim=2,
                     subset[a] = v
                 gone = {b for _, b in mpairs}
                 subset = [r for m, r in enumerate(subset) if m not in gone]
+                n_merged = len(gone)
 
         # -- limbs no existing person claimed start new persons (:166-177)
+        n_new = 0
         for k in range(kk):
             col = sum(msum[m][k] for m in range(mm))
             if col == 0:
@@ -376,6 +384,9 @@ def group_skeletons(limbs, skeleton, n_keypoints, person_thre, sort_dim=2,
                 new[jt, 0:4] = (row[3], row[4], row[5], row[12])
                 new[jf, 4] = new[jt, 4] = row[10]
                 subset.append(new)
+                n_new += 1
+        if trace is not None:
+            trace.append((li, mm, kk, n_new, n_merged))
 
     return delete_sort(subset, c, person_thre, sort_dim)
 
