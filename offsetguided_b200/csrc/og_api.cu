@@ -21,14 +21,6 @@ void set_error(const char *fmt, ...) {
     va_end(ap);
 }
 
-int chain_carveout_percent() {
-    static const int value = [] {
-        const char *env = getenv("OG_CARVEOUT");
-        return env ? atoi(env) : kChainCarveoutPercent;
-    }();
-    return value;
-}
-
 }  // namespace og
 
 using namespace og;
@@ -56,31 +48,10 @@ struct DevBuf {
     }
 };
 
-template <typename T>
-struct PinnedBuf {
-    T *ptr = nullptr;
-    size_t cap = 0;
-    int ensure(size_t need) {
-        if (need <= cap) return OG_OK;
-        if (ptr) OG_CUDA_TRY(cudaFreeHost(ptr));
-        ptr = nullptr;
-        cap = 0;
-        const size_t grow = need + need / 4;
-        OG_CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&ptr), grow * sizeof(T)));
-        cap = grow;
-        return OG_OK;
-    }
-    void release() {
-        if (ptr) cudaFreeHost(ptr);
-        ptr = nullptr;
-        cap = 0;
-    }
-};
-
 }  // namespace
 
 constexpr int kSlots = OG_MAX_IN_FLIGHT;   // decode calls that may be in flight before a fetch
-constexpr int kMaxChunks = 8;      // image ranges of one host-API call (copy / decode pipeline)
+constexpr int kMaxChunks = 4;      // image ranges of one host-API call (copy / decode pipeline)
 constexpr int kGraphsPerSlot = 4;  // captured device-path chains a result slot keeps
 // start, after prep, K1 pass 1 | select start, select = K2 start, K2, K3, end (see mark())
 constexpr int kStageEvents = 8;
@@ -194,9 +165,6 @@ struct og_handle {
     int device;
     int warp_rows;               // person-table rows of the one-warp-per-image K3 kernel (0 = off)
     int result_rows;             // pose rows per image the pinned result buffer starts with
-    int smem_rows;               // person-table rows of the CTA kernel, batches up to one image per SM
-    int smem_rows_dense;         // ... larger batches (several K3 CTAs per SM)
-    size_t group_smem;
     int64_t launches;
 
     // stand-alone stage APIs (og_nms_topk_f32, og_group_f32, ...): scratch in caller-stream order
@@ -220,9 +188,6 @@ struct og_handle {
     bool fused_enabled;
     bool graph_enabled;          // device path: replay a captured CUDA graph per slot
     bool zero_copy_enabled;      // host API: K2 gathers offsets straight from pinned host memory
-    int host_chunks;             // host API: image ranges of the copy / decode pipeline
-    int host_tail;               // ... with a short last range (tuning aid: OG_HOST_TAIL=0 disables)
-    int select_on_aux;           // host / full-resolution paths: 0 never, 1 fused path only, 2 always (tuning aid)
     int64_t fused_redos;
     int64_t k3_redos;            // fetches that ran the CTA grouping kernel for images the warp kernel gave up
     int64_t zero_copy_calls;
@@ -363,7 +328,6 @@ GroupLaunch group_launch(const og_handle *h, int n) {
     g.person_thre = c.person_thre;
     g.sort_dim = c.sort_dim;
     g.warp_rows = h->warp_rows;
-    g.smem_rows = n > h->sm_count ? h->smem_rows_dense : h->smem_rows;
     return g;
 }
 
@@ -598,7 +562,9 @@ int decode_range(og_handle *h, ResultSlot *slot, int chunk, int i0, int cn, cons
     // high-priority stream — the per-plane selection, K2 and K3 are latency-bound and occupy
     // a fraction of the SMs, so the next K1 pass (HBM-bound, on the caller's stream) overlaps
     // them instead of queueing behind them.
-    const bool sel_on_aux = chain || h->select_on_aux == 2 || (h->select_on_aux == 1 && fused != nullptr);
+    // On the full-resolution path the per-plane selection stays on the caller's stream: on the
+    // slot's stream it slows the next streaming pass down (profiles/r1_stream_sweep.txt).
+    const bool sel_on_aux = chain || fused != nullptr;
     if (!chain && sel_on_aux) {
         OG_CUDA_TRY(cudaEventRecord(slot->k1_done[chunk], k1s));
         OG_CUDA_TRY(cudaStreamWaitEvent(a, slot->k1_done[chunk], 0));
@@ -910,7 +876,6 @@ int og_create(const og_config *cfg, og_handle **out) {
     h->cp = nullptr;
     h->fused_enabled = true;
     h->graph_enabled = true;
-    if (const char *env = getenv("OG_GRAPH")) h->graph_enabled = atoi(env) != 0;     // tuning aid
     h->graph_replays = h->graph_builds = 0;
     h->k3_redos = 0;
     h->graph_clock = 0;
@@ -927,70 +892,37 @@ int og_create(const og_config *cfg, og_handle **out) {
     h->tables_version = 1;
     memset(&h->ft, 0, sizeof(h->ft));
     h->zero_copy_enabled = true;
-    h->host_chunks = 4;
-    if (const char *env = getenv("OG_HOST_CHUNKS")) {          // tuning aid
-        const int v = atoi(env);
-        if (v >= 1 && v <= kMaxChunks) h->host_chunks = v;
-    }
-    h->host_tail = 1;
-    if (const char *env = getenv("OG_HOST_TAIL")) h->host_tail = atoi(env) != 0;
-    h->select_on_aux = 1;
-    if (const char *env = getenv("OG_SELECT_ON_AUX")) h->select_on_aux = atoi(env);
     h->fused_redos = 0;
     h->zero_copy_calls = 0;
     h->tables_valid = false;
 
-    // person-table rows held in shared memory: as many as fit beside the work arrays
+    // Supported sizes: the CTA grouping kernel's shared work arrays for L * K persons plus a margin
+    // of 16 person rows (C * 24 bytes each) fit in 200 KB.  The kernel does not need the margin; it
+    // keeps the limit where the tests reach (the 64-keypoint ring at K = 96 is the largest such
+    // configuration), and a larger limit needs tests at the new sizes.
     GroupLaunch g = {};
     g.c = cfg->n_keypoints;
     g.l = cfg->n_limbs;
     g.k = cfg->topk;
     const int pmax = cfg->n_limbs * cfg->topk;
-    const size_t budget = std::min<size_t>(prop.sharedMemPerBlockOptin, 200 * 1024);
-    g.smem_rows = 0;
-    const size_t fixed = group_smem_bytes(g);
-    if (fixed + (size_t)16 * cfg->n_keypoints * 24 > budget) {
+    const size_t group_smem = group_smem_bytes(g);
+    const size_t supported = std::min<size_t>(prop.sharedMemPerBlockOptin, 200 * 1024);
+    if (group_smem + (size_t)16 * cfg->n_keypoints * 24 > supported) {
         delete h;
-        set_error("n_limbs * topk = %d needs %zu bytes of shared work arrays; unsupported", pmax, fixed);
+        set_error("n_limbs * topk = %d needs %zu bytes of shared work arrays; unsupported", pmax, group_smem);
         return OG_ERR_UNSUPPORTED;
     }
-    int rows = (int)((budget - fixed) / ((size_t)cfg->n_keypoints * 24));
-    rows = std::min(rows, std::min(pmax, 256));
-    // K3 is latency-bound (one CTA per image, issue slots ~4 % busy).  Up to one image per SM
-    // the large table is used: one CTA fills an SM's shared memory, which also spreads the CTAs
-    // over the SMs when they run beside the next call's K1.  Beyond that, several CTAs per SM
-    // multiply what an SM groups per second (profiles/r1_k3_occupancy_sweep.txt): the dense
-    // table keeps as many person rows as three (else two) CTAs per SM allow while ~40 KB of the
-    // SM stay L1 — but at least 64 rows: real scenes hold tens of persons, and a larger table
-    // restarts the image on the global slab.
-    int dense = rows;
-    for (const size_t share : {(size_t)62 * 1024, (size_t)94 * 1024}) {
-        if (fixed >= share) continue;
-        const int fit = (int)((share - fixed) / ((size_t)cfg->n_keypoints * 24));
-        if (fit >= 64) {
-            dense = std::min(rows, fit);
-            break;
-        }
-    }
-    if (const char *env = getenv("OG_K3_ROWS")) {              // tuning aid: person-table rows in shared memory
-        const int v = atoi(env);
-        if (v >= 16) rows = dense = std::min(rows, v);
-    }
-    h->smem_rows_dense = dense;
-    g.smem_rows = rows;
-    h->smem_rows = rows;
-    h->group_smem = group_smem_bytes(g);
     // One-warp-per-image kernel: 64 person rows (26 KB of shared memory for 17 keypoints, eight
     // images per SM) hold every real scene; an image that needs more is redone by the CTA kernel.
     h->warp_rows = std::min(64, pmax);
-    if (const char *env = getenv("OG_K3_WARP_ROWS")) {         // tuning aid; 0 = CTA kernel only
+    if (const char *env = getenv("OG_K3_WARP_ROWS")) {         // test aid; 0 = CTA kernel only
         const int v = atoi(env);
         if (v >= 0 && v <= 256) h->warp_rows = std::min(v, pmax);
     }
     g.warp_rows = h->warp_rows;
     while (g.warp_rows > 8 && group_warp_smem_bytes(g) > 96 * 1024) g.warp_rows /= 2;
     h->warp_rows = g.warp_rows;
-    int st = prepare_group_kernel(h->group_smem, group_warp_smem_bytes(g));
+    int st = prepare_group_kernel(group_smem, group_warp_smem_bytes(g));
     if (st != OG_OK) {
         delete h;
         return st;
@@ -998,7 +930,6 @@ int og_create(const og_config *cfg, og_handle **out) {
     {
         int least = 0, greatest = 0;
         cudaError_t err = cudaDeviceGetStreamPriorityRange(&least, &greatest);
-        if (const char *env = getenv("OG_AUX_PRIORITY")) if (atoi(env) == 0) greatest = least;   // tuning aid
         for (int i = 0; i < kSlots && err == cudaSuccess; ++i)
             err = cudaStreamCreateWithPriority(&h->slots[i].work, cudaStreamNonBlocking, greatest);
         if (err != cudaSuccess) {
@@ -1467,10 +1398,8 @@ int og_decode_features_host(og_handle *h, const float *hmp_host, const float *of
     int bounds[kMaxChunks + 1];
     int ranges = 0;
     {
-        const int chunks = std::max(1, std::min(h->host_chunks, kMaxChunks));
-        int tail = 0;
-        if (chunks >= 2 && n >= 16 && h->host_tail) tail = std::max(4, n / 16);
-        const int body = n - tail, body_ranges = tail ? chunks - 1 : chunks;
+        const int tail = n >= 16 ? std::max(4, n / 16) : 0;
+        const int body = n - tail, body_ranges = tail ? kMaxChunks - 1 : kMaxChunks;
         const int per = std::max((body + body_ranges - 1) / body_ranges, std::min(body, 4));
         bounds[0] = 0;
         for (int at = 0; at < body; at += per) bounds[++ranges] = std::min(at + per, body);

@@ -49,7 +49,6 @@ void set_error(const char *fmt, ...);
 // on the full-resolution path: K1 0.266 -> 0.305 ms when the kernel running beside it grew from
 // 2.5 to 10.5 KB of shared memory per CTA.  All chain kernels therefore ask for the same split.
 constexpr int kChainCarveoutPercent = 58;      // -> 132 KB shared memory, 96 KB L1 per SM
-int chain_carveout_percent();                  // kChainCarveoutPercent, or OG_CARVEOUT (tuning aid; -1 = leave the default)
 
 #ifdef __CUDACC__
 template <auto Kernel>
@@ -58,9 +57,8 @@ inline void prefer_chain_carveout() {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return;
     if ((done >> dev) & 1ull) return;
-    const int percent = chain_carveout_percent();
-    if (percent >= 0 &&
-        cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, percent) != cudaSuccess)
+    if (cudaFuncSetAttribute(Kernel, cudaFuncAttributePreferredSharedMemoryCarveout, kChainCarveoutPercent) !=
+        cudaSuccess)
         (void)cudaGetLastError();
     done |= 1ull << dev;
 }
@@ -240,8 +238,7 @@ struct GroupLaunch {
     double person_thre;
     int sort_dim;
     int warp_rows;              // person-table rows of the one-warp-per-image kernel (0 = skip it)
-    int smem_rows;              // person-table rows the CTA kernel keeps in shared memory
-    float *slab;                // global person tables, one per image (fallback)
+    float *slab;                // the CTA kernel's person tables, one per image
     size_t slab_stride;         // floats between images, multiple of 4
     int32_t *prep;              // group_prep_ints() ints: kept limb rows per (image, limb)
     float4 *rec;                // group_rec_vec4() float4: the kept rows themselves, compacted

@@ -31,8 +31,6 @@
 #include "og_common.cuh"
 #include "og_interp.cuh"
 
-#include <stdlib.h>
-
 #include <algorithm>
 
 namespace og {
@@ -431,12 +429,8 @@ int resident_per_sm(Kernel kernel) {
     return per_sm;
 }
 
-// tuning aids (read once): OG_K1F_CTAS_PER_SM caps the CTAs of the block kernel per SM (0 = all
-// that fit), OG_K1F_WAVES the CTA waves of its grid
-inline int env_int(const char *name, int fallback) {
-    const char *v = getenv(name);
-    return v ? atoi(v) : fallback;
-}
+// CTA waves of the block kernel's grid (2 and 1 measured no faster: profiles/r2_dropped_experiments.txt)
+constexpr int kCtaWaves = 4;
 
 template <typename T, int S, bool kCubic, bool kFlip>
 int launch_blocks_t(const T *hmp, size_t img_stride, int n_total, int h, int w, float thre,
@@ -447,12 +441,9 @@ int launch_blocks_t(const T *hmp, size_t img_stride, int n_total, int h, int w, 
     // (weights) is still amortised over several blocks, but CTAs retire during the kernel, so the
     // high-priority K3 CTAs of the previous call find room instead of waiting for a fully
     // persistent grid to drain.
-    static const int per_sm_fit = resident_per_sm(kernel);
-    static const int per_sm_cap = env_int("OG_K1F_CTAS_PER_SM", 0);
-    static const int waves = std::max(1, env_int("OG_K1F_WAVES", 4));
-    const int per_sm = per_sm_cap > 0 ? std::min(per_sm_cap, per_sm_fit) : per_sm_fit;
+    static const int per_sm = resident_per_sm(kernel);
     const int grid = (int)std::min<size_t>((blocks + kFusedThreads / 32 - 1) / (kFusedThreads / 32),
-                                           (size_t)sm_count * per_sm * waves);
+                                           (size_t)sm_count * per_sm * kCtaWaves);
     prefer_chain_carveout<fused_block_kernel<T, S, kCubic, kFlip>>();
     kernel<<<grid, kFusedThreads, 0, s>>>(hmp, img_stride, n_total, h, w, thre, block_list, n_active,
                                           cand_count, cand_keys);

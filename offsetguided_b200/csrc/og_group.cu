@@ -15,11 +15,12 @@
 //       has nobody to hide instruction fetches behind, and the unrolled body (58 KB of SASS)
 //       ran 5x slower than its dependent chain.  The person table is `warp_rows` rows
 //       of shared memory (26 KB for 64 rows x 17 joints), so eight images share an SM.
-//   group_kernel           one 256-thread CTA per image, table in shared memory or in a global
-//       slab of L*K rows: the images whose table outgrew the warp kernel's (noise inputs),
-//       flagged by it in `redo`; every other CTA of this launch exits at once.
+//   group_kernel           one 256-thread CTA per image, table in the image's global slab of
+//       L*K rows: the images whose table outgrew the warp kernel's (noise inputs), flagged by
+//       it in `redo`; every other CTA of this launch exits at once.
 //
-// The person table lives in shared memory as three planes per (person row, joint):
+// The person table (shared memory in the warp kernel, the slab in the CTA kernel) holds three
+// planes per (person row, joint):
 //   ids   int32   global keypoint id (-1 = unset)          pose column 5
 //   score float   best limb score seen for the joint       pose column 4
 //   xyvs  float4  x, y, keypoint score, keypoint scale     pose columns 0..3
@@ -37,9 +38,8 @@
 //       writes
 //   (4) append unclaimed limbs as new persons, using the reference's column-sum rule
 //       including its (-1)+(+1) cancellation quirk (group.py:166).
-// The table has `smem_rows` rows; if an image needs more (never seen outside noise inputs)
-// the same CTA restarts that image with the table in a global slab of L*K rows, which cannot
-// overflow (every new person consumes one limb row).
+// The slab cannot overflow: every new person consumes one kept limb row, and there are at most
+// L*K of those.
 #include "og_common.cuh"
 #include "og_prep.cuh"
 
@@ -79,7 +79,6 @@ struct GroupArgs {
     SkeletonDev sk;
     double person_thre;
     int sort_dim;
-    int smem_rows;
     int warp_rows;
     float *slab;     // per image: xyvs float4[PMAX*C], score float[PMAX*C], ids int[PMAX*C]
     size_t slab_stride;
@@ -133,17 +132,14 @@ group_prepare_kernel(const float *__restrict__ limbs, int L, int K, float dist_m
 // grouping
 // ---------------------------------------------------------------------------
 struct Layout {
-    size_t xyvs, score, ids, conn, rows, k_int, p_i32, p_i16, p_u8, p_f64, warp, flags, total;
+    size_t conn, rows, k_int, p_i32, p_i16, p_u8, p_f64, warp, flags, total;
 };
 
 // k_int: 6 int arrays of K; p_i32: 3 int arrays of PMAX; p_i16: 3 int16 arrays of PMAX
-__host__ __device__ inline Layout make_layout(int C, int L, int K, int smem_rows) {
+__host__ __device__ inline Layout make_layout(int L, int K) {
     const size_t pmax = (size_t)L * K;
     Layout lo;
     size_t at = 0;
-    lo.xyvs = at;  at += (size_t)smem_rows * C * 16;
-    lo.score = at; at += (size_t)smem_rows * C * 4;
-    lo.ids = at;   at += (size_t)smem_rows * C * 4;
     lo.conn = at;  at += 2 * align_up((size_t)K * OG_LIMB_COLS * 4, 16);     // double buffer
     lo.rows = at;  at += 2 * align_up((size_t)(K + 1) * 4, 16);               // kept rows + count
     lo.k_int = at; at += (size_t)6 * K * 4;
@@ -227,7 +223,7 @@ group_kernel(GroupArgs a, const float *__restrict__ limbs, const int32_t *__rest
 #endif
     const int C = a.C, L = a.L, K = a.K;
     const int pmax = L * K;
-    const Layout lo = make_layout(C, L, K, a.smem_rows);
+    const Layout lo = make_layout(L, K);
     const int tid = threadIdx.x, T = blockDim.x;
     const int lane = tid & 31, wid = tid >> 5;
     const int img = blockIdx.x;
@@ -261,212 +257,188 @@ group_kernel(GroupArgs a, const float *__restrict__ limbs, const int32_t *__rest
     const float *limbs_img = limbs + (size_t)img * L * K * OG_LIMB_COLS;
     const int32_t *prep_img = prep + (size_t)img * L * (K + 1);
 
-    float4 *xyvs = nullptr;
-    float *score = nullptr;
-    int *ids = nullptr;
-    int mm = 0;
+    float *slab_img = a.slab + (size_t)img * a.slab_stride;
+    float4 *xyvs = reinterpret_cast<float4 *>(slab_img);
+    float *score = slab_img + (size_t)pmax * C * 4;
+    int *ids = reinterpret_cast<int *>(slab_img + (size_t)pmax * C * 5);
+    int mm = 0, nalloc = 0;
 
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        int pcap;
-        if (attempt == 0) {
-            xyvs = reinterpret_cast<float4 *>(smem + lo.xyvs);
-            score = reinterpret_cast<float *>(smem + lo.score);
-            ids = reinterpret_cast<int *>(smem + lo.ids);
-            pcap = a.smem_rows;
-        } else {
-            float *base = a.slab + (size_t)img * a.slab_stride;
-            xyvs = reinterpret_cast<float4 *>(base);
-            score = base + (size_t)pmax * C * 4;
-            ids = reinterpret_cast<int *>(base + (size_t)pmax * C * 5);
-            pcap = pmax;
-        }
-        mm = 0;
-        int nalloc = 0;
-        bool overflow = false;
+    // rows and kept list of limb type li + 1 are fetched with cp.async while type li runs
+    auto fetch_rows = [&](int li_next) {
+        float *dst = s_conn_buf[li_next & 1];
+        const float *src = limbs_img + (size_t)li_next * K * OG_LIMB_COLS;
+        for (int i = tid; i < K * OG_LIMB_COLS; i += T) cp_async4(dst + i, src + i);
+        int *rdst = s_rows_buf[li_next & 1];
+        const int32_t *rsrc = prep_img + (size_t)li_next * (K + 1);
+        for (int i = tid; i <= K; i += T) cp_async4(rdst + i, rsrc + i);
+        asm volatile("cp.async.commit_group;");
+    };
+    fetch_rows(0);
+    for (int li = 0; li < L; ++li) {
+        const int jf = a.sk.from[li], jt = a.sk.to[li];
+        const float *s_conn = s_conn_buf[li & 1];
+        const int *s_rows = s_rows_buf[li & 1];
+        asm volatile("cp.async.wait_all;" ::: "memory");        // data of type li has landed
+        if (tid < kNumFlags) s_flag[tid] = 0;
         __syncthreads();
+        // The buffers of type li + 1 are those of type li - 1: only after the barrier has every
+        // thread finished reading them (a type with kk == 0 leaves its iteration without one).
+        if (li + 1 < L) fetch_rows(li + 1);
+        OG_K3_PROF(0);
+        const int kk = s_rows[K];
+        if (kk == 0) continue;                                         // group.py:84-85
 
-        // rows and kept list of limb type li + 1 are fetched with cp.async while type li runs
-        auto fetch_rows = [&](int li_next) {
-            float *dst = s_conn_buf[li_next & 1];
-            const float *src = limbs_img + (size_t)li_next * K * OG_LIMB_COLS;
-            for (int i = tid; i < K * OG_LIMB_COLS; i += T) cp_async4(dst + i, src + i);
-            int *rdst = s_rows_buf[li_next & 1];
-            const int32_t *rsrc = prep_img + (size_t)li_next * (K + 1);
-            for (int i = tid; i <= K; i += T) cp_async4(rdst + i, rsrc + i);
-            asm volatile("cp.async.commit_group;");
-        };
-        fetch_rows(0);
-        for (int li = 0; li < L && !overflow; ++li) {
-            const int jf = a.sk.from[li], jt = a.sk.to[li];
-            const float *s_conn = s_conn_buf[li & 1];
-            const int *s_rows = s_rows_buf[li & 1];
-            asm volatile("cp.async.wait_all;" ::: "memory");        // data of type li has landed
-            if (tid < kNumFlags) s_flag[tid] = 0;
-            __syncthreads();
-            // The buffers of type li + 1 are those of type li - 1: only after the barrier has every
-            // thread finished reading them (a type with kk == 0 leaves its iteration without one).
-            if (li + 1 < L) fetch_rows(li + 1);
-            OG_K3_PROF(0);
-            const int kk = s_rows[K];
-            if (kk == 0) continue;                                         // group.py:84-85
-
-            // ---- stage ids / scores of the kept rows; reset the per-person match slots
-            for (int j = tid; j < kk; j += T) {
-                const float *r = s_conn + s_rows[j] * OG_LIMB_COLS;
-                s_kind1[j] = (int)r[6];
-                s_kind2[j] = (int)r[7];
-                s_kscore[j] = r[10];
-                s_n1[j] = 0;
-                s_n2[j] = 0;
-            }
-            for (int m = tid; m < mm; m += T) {
-                s_pk1[m] = -1;
-                s_pk2[m] = -1;
-                s_blast[m] = -1;
-                s_del[m] = 0;
-            }
-            __syncthreads();
-            OG_K3_PROF(1);
-            // ---- match persons x kept limbs on the pre-update snapshot (group.py:87-109),
-            //      one thread per pair; the last matching limb of a person wins (atomicMax)
-            for (int e = tid; e < mm * kk; e += T) {
-                const int m = e / kk, j = e - m * kk;
-                const int row = s_order[m];
-                const int ms = (ids[row * C + jf] == s_kind1[j] ? 1 : 0) +
-                               (ids[row * C + jt] == s_kind2[j] ? 1 : 0);
-                if (ms == 0) continue;
-                const float sc = s_kscore[j];
-                const bool rep = (sc > score[row * C + jt]) || (sc > score[row * C + jf]);
-                if (ms == 2) {
-                    atomicAdd(&s_n2[j], 1);
-                    if (rep) {
-                        atomicMax(&s_pk2[m], j);
-                        s_flag[kAnyP2] = 1;
-                    }
-                } else {
-                    atomicAdd(&s_n1[j], 1);
-                    if (rep) {
-                        atomicMax(&s_pk1[m], j);
-                        s_flag[kAnyP1] = 1;
-                    }
-                }
-            }
-            __syncthreads();
-            OG_K3_PROF(2);
-            // ---- apply: both ends known (group.py:114-119), then one end known (:124-135)
-            for (int m = tid; m < mm; m += T) {
-                const int row = s_order[m];
-                const int k2 = s_pk2[m];
-                if (k2 >= 0) {
-                    const float sc = s_kscore[k2];
-                    score[row * C + jf] = fmaxf(sc, score[row * C + jf]);
-                    score[row * C + jt] = fmaxf(sc, score[row * C + jt]);
-                }
-                const int k1 = s_pk1[m];
-                if (k1 >= 0) {
-                    const float *r = s_conn + s_rows[k1] * OG_LIMB_COLS;
-                    ids[row * C + jf] = s_kind1[k1];
-                    ids[row * C + jt] = s_kind2[k1];
-                    xyvs[row * C + jf] = make_float4(r[0], r[1], r[2], r[11]);
-                    xyvs[row * C + jt] = make_float4(r[3], r[4], r[5], r[12]);
-                    const float sc = s_kscore[k1];
-                    score[row * C + jf] = fmaxf(sc, score[row * C + jf]);
-                    score[row * C + jt] = fmaxf(sc, score[row * C + jt]);
-                }
-            }
-            __syncthreads();
-            OG_K3_PROF(3);
-            // ---- merge persons sharing exactly two keypoint ids (group.py:140-155), one thread
-            //      per ordered pair p < q; the largest partner of p wins
-            int mm_after = mm;
-            if (mm >= 2) {
-                for (int e = tid; e < mm * mm; e += T) {
-                    const int p = e / mm, q = e - p * mm;
-                    if (q <= p) continue;
-                    const int rowa = s_order[p], rowb = s_order[q];
-                    int cnt = 0;
-                    for (int c = 0; c < C; ++c) {
-                        const int ia = ids[rowa * C + c];
-                        cnt += (ia != -1 && ia == ids[rowb * C + c]) ? 1 : 0;
-                    }
-                    if (cnt == 2) {
-                        atomicMax(&s_blast[p], q);
-                        s_del[q] = 1;
-                        s_flag[kAnyMerge] = 1;
-                    }
-                }
-                __syncthreads();
-                OG_K3_PROF(4);
-                if (s_flag[kAnyMerge]) {
-                    for (int p = tid; p < mm; p += T) {
-                        const int q = s_blast[p];
-                        if (q < 0 || s_del[p]) continue;      // deleted rows are never read again
-                        const int rowa = s_order[p], rowb = s_order[q];
-                        for (int c = 0; c < C; ++c) {
-                            ids[rowa * C + c] = max(ids[rowa * C + c], ids[rowb * C + c]);
-                            score[rowa * C + c] = fmaxf(score[rowa * C + c], score[rowb * C + c]);
-                            xyvs[rowa * C + c] = max4(xyvs[rowa * C + c], xyvs[rowb * C + c]);
-                        }
-                    }
-                    mm_after = block_scan(mm, [&](int p) { return s_del[p] == 0; }, s_pos, s_warp);
-                    for (int p = tid; p < mm; p += T)
-                        if (!s_del[p]) s_order2[s_pos[p]] = s_order[p];
-                    __syncthreads();
-                    int16_t *tmp = s_order;
-                    s_order = s_order2;
-                    s_order2 = tmp;
-                }
-            }
-            // ---- warp 0: unclaimed limbs start new persons (group.py:166-177), column-sum
-            //      rule with its (-1) + (+1) cancellation
-            if (wid == 0) {
-                const int w2 = s_flag[kAnyP2] ? -1 : 2;
-                const int w1 = s_flag[kAnyP1] ? -1 : 1;
-                int nnew = 0;
-                for (int j0 = 0; j0 < kk; j0 += 32) {
-                    const int j = j0 + lane;
-                    const bool isnew = j < kk && (s_n2[j] * w2 + s_n1[j] * w1 == 0);
-                    const unsigned mask = __ballot_sync(0xffffffffu, isnew);
-                    if (isnew) s_new[nnew + __popc(mask & ((1u << lane) - 1u))] = j;
-                    nnew += __popc(mask);
-                }
-                if (lane == 0) s_flag[kNNew] = nnew;
-            }
-            __syncthreads();
-            OG_K3_PROF(5);
-            const int nnew = s_flag[kNNew];
-            if (nalloc + nnew > pcap) {
-                overflow = true;          // uniform: restart this image on the global slab
-                continue;
-            }
-            for (int e = tid; e < nnew * C; e += T) {
-                const int q = e / C, c = e - q * C;
-                const int j = s_new[q];
-                const int at = (nalloc + q) * C + c;
-                const float *r = s_conn + s_rows[j] * OG_LIMB_COLS;
-                if (c == 0) s_order[mm_after + q] = (int16_t)(nalloc + q);
-                if (c == jt) {
-                    ids[at] = s_kind2[j];
-                    xyvs[at] = make_float4(r[3], r[4], r[5], r[12]);
-                    score[at] = s_kscore[j];
-                } else if (c == jf) {
-                    ids[at] = s_kind1[j];
-                    xyvs[at] = make_float4(r[0], r[1], r[2], r[11]);
-                    score[at] = s_kscore[j];
-                } else {
-                    ids[at] = -1;
-                    xyvs[at] = make_float4(-1.f, -1.f, -1.f, -1.f);
-                    score[at] = -1.0f;
-                }
-            }
-            nalloc += nnew;
-            mm = mm_after + nnew;
-            __syncthreads();
-            OG_K3_PROF(6);
+        // ---- stage ids / scores of the kept rows; reset the per-person match slots
+        for (int j = tid; j < kk; j += T) {
+            const float *r = s_conn + s_rows[j] * OG_LIMB_COLS;
+            s_kind1[j] = (int)r[6];
+            s_kind2[j] = (int)r[7];
+            s_kscore[j] = r[10];
+            s_n1[j] = 0;
+            s_n2[j] = 0;
         }
-        asm volatile("cp.async.wait_all;" ::: "memory");
-        if (!overflow) break;
+        for (int m = tid; m < mm; m += T) {
+            s_pk1[m] = -1;
+            s_pk2[m] = -1;
+            s_blast[m] = -1;
+            s_del[m] = 0;
+        }
+        __syncthreads();
+        OG_K3_PROF(1);
+        // ---- match persons x kept limbs on the pre-update snapshot (group.py:87-109),
+        //      one thread per pair; the last matching limb of a person wins (atomicMax)
+        for (int e = tid; e < mm * kk; e += T) {
+            const int m = e / kk, j = e - m * kk;
+            const int row = s_order[m];
+            const int ms = (ids[row * C + jf] == s_kind1[j] ? 1 : 0) +
+                           (ids[row * C + jt] == s_kind2[j] ? 1 : 0);
+            if (ms == 0) continue;
+            const float sc = s_kscore[j];
+            const bool rep = (sc > score[row * C + jt]) || (sc > score[row * C + jf]);
+            if (ms == 2) {
+                atomicAdd(&s_n2[j], 1);
+                if (rep) {
+                    atomicMax(&s_pk2[m], j);
+                    s_flag[kAnyP2] = 1;
+                }
+            } else {
+                atomicAdd(&s_n1[j], 1);
+                if (rep) {
+                    atomicMax(&s_pk1[m], j);
+                    s_flag[kAnyP1] = 1;
+                }
+            }
+        }
+        __syncthreads();
+        OG_K3_PROF(2);
+        // ---- apply: both ends known (group.py:114-119), then one end known (:124-135)
+        for (int m = tid; m < mm; m += T) {
+            const int row = s_order[m];
+            const int k2 = s_pk2[m];
+            if (k2 >= 0) {
+                const float sc = s_kscore[k2];
+                score[row * C + jf] = fmaxf(sc, score[row * C + jf]);
+                score[row * C + jt] = fmaxf(sc, score[row * C + jt]);
+            }
+            const int k1 = s_pk1[m];
+            if (k1 >= 0) {
+                const float *r = s_conn + s_rows[k1] * OG_LIMB_COLS;
+                ids[row * C + jf] = s_kind1[k1];
+                ids[row * C + jt] = s_kind2[k1];
+                xyvs[row * C + jf] = make_float4(r[0], r[1], r[2], r[11]);
+                xyvs[row * C + jt] = make_float4(r[3], r[4], r[5], r[12]);
+                const float sc = s_kscore[k1];
+                score[row * C + jf] = fmaxf(sc, score[row * C + jf]);
+                score[row * C + jt] = fmaxf(sc, score[row * C + jt]);
+            }
+        }
+        __syncthreads();
+        OG_K3_PROF(3);
+        // ---- merge persons sharing exactly two keypoint ids (group.py:140-155), one thread
+        //      per ordered pair p < q; the largest partner of p wins
+        int mm_after = mm;
+        if (mm >= 2) {
+            for (int e = tid; e < mm * mm; e += T) {
+                const int p = e / mm, q = e - p * mm;
+                if (q <= p) continue;
+                const int rowa = s_order[p], rowb = s_order[q];
+                int cnt = 0;
+                for (int c = 0; c < C; ++c) {
+                    const int ia = ids[rowa * C + c];
+                    cnt += (ia != -1 && ia == ids[rowb * C + c]) ? 1 : 0;
+                }
+                if (cnt == 2) {
+                    atomicMax(&s_blast[p], q);
+                    s_del[q] = 1;
+                    s_flag[kAnyMerge] = 1;
+                }
+            }
+            __syncthreads();
+            OG_K3_PROF(4);
+            if (s_flag[kAnyMerge]) {
+                for (int p = tid; p < mm; p += T) {
+                    const int q = s_blast[p];
+                    if (q < 0 || s_del[p]) continue;      // deleted rows are never read again
+                    const int rowa = s_order[p], rowb = s_order[q];
+                    for (int c = 0; c < C; ++c) {
+                        ids[rowa * C + c] = max(ids[rowa * C + c], ids[rowb * C + c]);
+                        score[rowa * C + c] = fmaxf(score[rowa * C + c], score[rowb * C + c]);
+                        xyvs[rowa * C + c] = max4(xyvs[rowa * C + c], xyvs[rowb * C + c]);
+                    }
+                }
+                mm_after = block_scan(mm, [&](int p) { return s_del[p] == 0; }, s_pos, s_warp);
+                for (int p = tid; p < mm; p += T)
+                    if (!s_del[p]) s_order2[s_pos[p]] = s_order[p];
+                __syncthreads();
+                int16_t *tmp = s_order;
+                s_order = s_order2;
+                s_order2 = tmp;
+            }
+        }
+        // ---- warp 0: unclaimed limbs start new persons (group.py:166-177), column-sum
+        //      rule with its (-1) + (+1) cancellation
+        if (wid == 0) {
+            const int w2 = s_flag[kAnyP2] ? -1 : 2;
+            const int w1 = s_flag[kAnyP1] ? -1 : 1;
+            int nnew = 0;
+            for (int j0 = 0; j0 < kk; j0 += 32) {
+                const int j = j0 + lane;
+                const bool isnew = j < kk && (s_n2[j] * w2 + s_n1[j] * w1 == 0);
+                const unsigned mask = __ballot_sync(0xffffffffu, isnew);
+                if (isnew) s_new[nnew + __popc(mask & ((1u << lane) - 1u))] = j;
+                nnew += __popc(mask);
+            }
+            if (lane == 0) s_flag[kNNew] = nnew;
+        }
+        __syncthreads();
+        OG_K3_PROF(5);
+        const int nnew = s_flag[kNNew];
+        for (int e = tid; e < nnew * C; e += T) {
+            const int q = e / C, c = e - q * C;
+            const int j = s_new[q];
+            const int at = (nalloc + q) * C + c;
+            const float *r = s_conn + s_rows[j] * OG_LIMB_COLS;
+            if (c == 0) s_order[mm_after + q] = (int16_t)(nalloc + q);
+            if (c == jt) {
+                ids[at] = s_kind2[j];
+                xyvs[at] = make_float4(r[3], r[4], r[5], r[12]);
+                score[at] = s_kscore[j];
+            } else if (c == jf) {
+                ids[at] = s_kind1[j];
+                xyvs[at] = make_float4(r[0], r[1], r[2], r[11]);
+                score[at] = s_kscore[j];
+            } else {
+                ids[at] = -1;
+                xyvs[at] = make_float4(-1.f, -1.f, -1.f, -1.f);
+                score[at] = -1.0f;
+            }
+        }
+        nalloc += nnew;
+        mm = mm_after + nnew;
+        __syncthreads();
+        OG_K3_PROF(6);
     }
+    asm volatile("cp.async.wait_all;" ::: "memory");
 
     // ---- person score, threshold, stable descending sort (group.py:188-219)
     for (int m = tid; m < mm; m += T) {
@@ -1168,7 +1140,6 @@ GroupArgs to_args(const GroupLaunch &g) {
     a.sk = g.sk;
     a.person_thre = g.person_thre;
     a.sort_dim = g.sort_dim;
-    a.smem_rows = g.smem_rows;
     a.warp_rows = g.warp_rows;
     a.slab = g.slab;
     a.slab_stride = g.slab_stride;
@@ -1195,7 +1166,7 @@ int read_k3_profile(unsigned long long *out16, bool reset) {
 #endif
 }
 
-size_t group_smem_bytes(const GroupLaunch &g) { return make_layout(g.c, g.l, g.k, g.smem_rows).total; }
+size_t group_smem_bytes(const GroupLaunch &g) { return make_layout(g.l, g.k).total; }
 
 size_t group_warp_smem_bytes(const GroupLaunch &g) {
     return g.warp_rows > 0 ? make_warp_layout(g.c, g.l, g.k, g.warp_rows).total : 0;
@@ -1257,19 +1228,10 @@ int launch_group_redo(const GroupLaunch &g, const float *limbs, float *out_poses
     if (g.n == 0) return OG_OK;
     GroupLaunch cta = g;
     cta.lazy_flag = nullptr;
-    const int32_t *redo = nullptr;
-    if (g.warp_rows > 0) {
-        redo = g.redo;
-        // Behind the warp kernel the CTA kernel only redoes images whose table outgrew the warp
-        // kernel's rows, and nearly every CTA of this launch exits at once: it gets NO shared-memory
-        // table (the image goes straight to its global slab), so that a launch of early-exit CTAs
-        // does not ask every SM for 200 KB of shared memory while the next call's streaming
-        // kernels are resident.
-        cta.smem_rows = 0;
-        prefer_chain_carveout<group_kernel>();      // early-exit launch: blend in
-    }
-    group_kernel<<<g.n, kGroupThreads, group_smem_bytes(cta), s>>>(
-        to_args(cta), limbs, g.prep, out_poses, capacity_rows, out_offset, out_count, out_total, redo);
+    prefer_chain_carveout<group_kernel>();
+    group_kernel<<<g.n, kGroupThreads, group_smem_bytes(g), s>>>(
+        to_args(cta), limbs, g.prep, out_poses, capacity_rows, out_offset, out_count, out_total,
+        g.warp_rows > 0 ? g.redo : nullptr);
     OG_CUDA_TRY(cudaGetLastError());
     if (launches) *launches += 1;
     return OG_OK;

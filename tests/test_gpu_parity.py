@@ -197,8 +197,8 @@ def test_k3_on_reference_limbs_bit_exact(cuda_device, name):
 
 
 def test_k3_random_tables_against_oracle(cuda_device):
-    """Fresh seeded fuzz (not from the fixture), incl. pure-noise tables that overflow the
-    shared-memory person table and restart on the global slab."""
+    """Fresh seeded fuzz (not from the fixture), incl. pure-noise tables that outgrow the warp
+    kernel's person table and are regrouped by the CTA kernel."""
     rng = np.random.RandomState(77)
     skel = cfg.COCO_PERSON_SKELETON
     for case in range(40):
@@ -220,15 +220,14 @@ def test_k3_random_tables_against_oracle(cuda_device):
         assert got.shape == ref.shape and np.array_equal(got, ref), f'case {case} k={k} pool={pool}'
 
 
-def test_k3_large_batch_uses_dense_tables(cuda_device):
-    """Beyond one image per SM K3 keeps a smaller person table in shared memory (three CTAs per
-    SM); every image — also the ones whose table overflows it and restarts on the global slab —
-    must come out as in a small batch."""
+def test_k3_large_batch_with_warp_overflow_against_oracle(cuda_device):
+    """A batch of 400 images, some of whose tables outgrow the warp kernel's person table and are
+    regrouped by the CTA kernel: every image equals the oracle, as in a batch of 12."""
     rng = np.random.RandomState(123)
     skel = cfg.COCO_PERSON_SKELETON
     tables = []
     for case in range(12):
-        k, pool = 32, int(rng.choice([4, 10, 400]))         # pool 400: ~100+ persons, overflows 100 rows
+        k, pool = 32, int(rng.choice([4, 10, 400]))         # pool 400: ~100+ persons, outgrows 64 rows
         limbs = np.zeros((19, k, 13), np.float32)
         xy = rng.randint(1, 600, size=(17, pool, 2)).astype(np.float32)
         ids = rng.randint(0, 640 * 640, size=(17, pool))

@@ -302,7 +302,7 @@ def _group(monkeypatch, warp_rows, skel, c, stack):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize('rows', [64, 128])
-@pytest.mark.parametrize('batch', [100, 400])          # one image per SM or fewer / several
+@pytest.mark.parametrize('batch', [100, 400])          # fewer images than SMs / several per SM
 def test_crowd_tables_warp_cta_and_oracles(cuda_device, monkeypatch, rows, batch):
     tables, traces = _crowd_tables(), _traces('crowd')
     groups = {}
@@ -444,9 +444,9 @@ def test_crowd_scenes_end_to_end(cuda_device, monkeypatch, template, topk):
 
 @pytest.mark.gpu
 def test_ring_64_keypoints_at_largest_k(cuda_device):
-    """64 keypoints / 64 limbs (a ring) at K = 96, the largest top-K whose CTA-kernel work arrays
-    (L * K persons) fit: the warp kernel's table is halved to 32 rows to fit 96 KB of shared
-    memory, so 24 persons stay in it and 40 go to the CTA kernel."""
+    """64 keypoints / 64 limbs (a ring) at K = 96, the largest top-K the library accepts for this
+    skeleton (K = 97 is refused): the warp kernel's table is halved to 32 rows to fit 96 KB of
+    shared memory, so 24 persons stay in it and 40 go to the CTA kernel."""
     import torch
     from offsetguided_b200 import _lib
     from offsetguided_b200.engine import DecoderEngine
