@@ -17,7 +17,8 @@
  *   - every function returns an og_status (0 = OG_OK); og_last_error() gives the
  *     text of the last failure on the calling thread;
  *   - all maps are float32, NCHW, contiguous (og_decode_features_dev_ex also takes
- *     bfloat16 / float16 maps and image-strided views); "dev" pointers are device
+ *     bfloat16 / float16 maps and image-strided views, og_decode_features_dev_strided
+ *     channels-last ones as well); "dev" pointers are device
  *     memory of the handle's GPU, "host" pointers are host memory (pinned memory makes
  *     the copies asynchronous and lets the offset maps stay on the host);
  *   - `stream` is the caller's stream: inputs are consumed in its order.  A handle owns one
@@ -218,13 +219,34 @@ int og_decode_features_dev(og_handle *h, const float *hmp_dev, const float *off_
  * of one packed [n, C + 2L, h, w] head output are decoded in place, without a split or a
  * float32 copy.  bf16 / f16 values widen exactly to float32: results are bit-identical to
  * decoding the converted maps.  Fused path only (strides 2 / 4 / 8, thre_hmp > 0); the exact redo of a
- * candidate overflow converts the maps to dense float32 on the device first. */
+ * candidate overflow converts the maps to dense float32 on the device first.  Equivalent to
+ * og_decode_features_dev_strided with planar strides. */
 int og_decode_features_dev_ex(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
                               int64_t hmp_image_stride, int64_t off_image_stride,
                               int n, int hgt, int w, int hmp_stride, int off_stride,
                               int resize_mode, int flip_test,
                               const int32_t *kp_flip, const int32_t *limb_flip,
                               const int32_t *limb_reserve, int n_reserve, void *stream);
+
+/* og_decode_features_dev_ex for maps in either memory layout, such as the outputs of a network run
+ * in PyTorch's channels_last format, decoded in place without a transposing copy.  Each map is
+ * described by its element strides in (image, channel, row, column) order, as Tensor.stride()
+ * reports them; the two maps are classified independently:
+ *   planar         (s_n, hgt * w, w, 1), s_n >= channels * hgt * w;
+ *   channels-last  (s_n, 1, w * p, p), p >= channels (p = channel count of the whole packed tensor,
+ *                  the base pointer may sit at any element), s_n >= hgt * w * p.
+ * s_n is not checked when the buffer holds one image; a layout that is both is planar.  Any other
+ * strides return OG_ERR_INVALID_ARGUMENT before anything is launched.  Channels-last heat maps are
+ * read once by a transposing scan that writes them, flip-fused, as dense float32 planes into a
+ * scratch buffer of the result slot (n * C * hgt * w * 4 bytes, allocated by the first such call);
+ * results are bit-identical to decoding contiguous float32 copies.  Fused path only, like
+ * og_decode_features_dev_ex. */
+int og_decode_features_dev_strided(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
+                                   const int64_t hmp_elem_strides[4], const int64_t off_elem_strides[4],
+                                   int n, int hgt, int w, int hmp_stride, int off_stride,
+                                   int resize_mode, int flip_test,
+                                   const int32_t *kp_flip, const int32_t *limb_flip,
+                                   const int32_t *limb_reserve, int n_reserve, void *stream);
 
 /* og_decode_features_dev with the optional heads and flags of PostProcess.generate_poses
  * (decoder/factory.py:52-96, collect.py:111-138, 158-165, 213-218), still on the fused path: the
@@ -245,12 +267,19 @@ int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float
 /* A prepared og_decode_features_dev_ex: a network writes its outputs to the same buffers batch
  * after batch, so a caller validates and records the arguments once (og_plan_features, which
  * also installs the flip tables) and then launches each batch with three arguments.  A plan stays
- * valid for the life of the handle while the buffers exist and the flip tables are unchanged. */
+ * valid for the life of the handle while the buffers exist and the flip tables are unchanged.
+ * The strides are validated when the plan is made. */
 int og_plan_features(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
                      int64_t hmp_image_stride, int64_t off_image_stride, int n, int hgt, int w,
                      int hmp_stride, int off_stride, int resize_mode, int flip_test,
                      const int32_t *kp_flip, const int32_t *limb_flip, const int32_t *limb_reserve,
                      int n_reserve, int32_t *plan_id);
+/* og_plan_features for og_decode_features_dev_strided: planar or channels-last maps. */
+int og_plan_features_strided(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
+                             const int64_t hmp_elem_strides[4], const int64_t off_elem_strides[4],
+                             int n, int hgt, int w, int hmp_stride, int off_stride, int resize_mode,
+                             int flip_test, const int32_t *kp_flip, const int32_t *limb_flip,
+                             const int32_t *limb_reserve, int n_reserve, int32_t *plan_id);
 int og_plan_launch(og_handle *h, int32_t plan_id, void *stream);
 
 /* Up to OG_MAX_IN_FLIGHT og_decode_* calls may be in flight on a handle (results are queued in

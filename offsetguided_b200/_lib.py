@@ -62,6 +62,7 @@ class OgError(RuntimeError):
 
 _vp = ctypes.c_void_p
 _i = ctypes.c_int
+_i64_p = ctypes.POINTER(ctypes.c_int64)
 # name -> (restype, argtypes); every symbol include/og_decoder.h declares
 SIGNATURES = {
     'og_last_error': (ctypes.c_char_p, []),
@@ -88,12 +89,16 @@ SIGNATURES = {
                                     c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
     'og_decode_features_dev_ex': (_i, [_vp, _vp, _vp, _i, ctypes.c_int64, ctypes.c_int64, _i, _i, _i, _i, _i,
                                        _i, _i, c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
+    'og_decode_features_dev_strided': (_i, [_vp, _vp, _vp, _i, _i64_p, _i64_p, _i, _i, _i, _i, _i, _i, _i,
+                                            c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
     'og_fetch_poses': (_i, [_vp, ctypes.POINTER(c_float_p), ctypes.POINTER(c_int32_p),
                             ctypes.POINTER(c_int32_p), ctypes.POINTER(ctypes.c_int32)]),
     'og_decode_features_heads_dev': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i,
                                           _i, _i, c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
     'og_plan_features': (_i, [_vp, _vp, _vp, _i, ctypes.c_int64, ctypes.c_int64, _i, _i, _i, _i, _i,
                               _i, _i, c_int32_p, c_int32_p, c_int32_p, _i, ctypes.POINTER(ctypes.c_int32)]),
+    'og_plan_features_strided': (_i, [_vp, _vp, _vp, _i, _i64_p, _i64_p, _i, _i, _i, _i, _i, _i, _i,
+                                      c_int32_p, c_int32_p, c_int32_p, _i, ctypes.POINTER(ctypes.c_int32)]),
     'og_plan_launch': (_i, [_vp, ctypes.c_int32, _vp]),
     'og_fetch_result': (_i, [_vp, ctypes.POINTER(OgResult)]),
     'og_set_frames': (_i, [_vp, ctypes.POINTER(ctypes.c_double), _i]),
@@ -141,6 +146,11 @@ def check(status):
         lib = load()
         raise OgError('%s: %s' % (lib.og_status_string(status).decode(),
                                   lib.og_last_error().decode()))
+
+
+def int64_array(values):
+    values = [int(v) for v in values]
+    return (ctypes.c_int64 * max(len(values), 1))(*values)
 
 
 def int32_array(values):

@@ -78,6 +78,7 @@ struct GraphKey {
     const void *hmp, *off;
     int dtype;
     size_t hmp_image_stride, off_image_stride;
+    size_t hmp_plane_stride, hmp_pixel_stride, off_plane_stride, off_pixel_stride;   // planar or channels-last
     int n, hgt, w, stride, mode, flip, coco;
     uint64_t tables_version, buffers_version;
     const void *scale, *jitter;             // optional heads (og_decode_features_heads_dev)
@@ -85,7 +86,9 @@ struct GraphKey {
     bool operator==(const GraphKey &o) const {
         return hmp == o.hmp && off == o.off && dtype == o.dtype && coco == o.coco && hmp_image_stride == o.hmp_image_stride &&
                scale == o.scale && jitter == o.jitter && vector_nd == o.vector_nd && use_jitter == o.use_jitter &&
-               off_image_stride == o.off_image_stride && n == o.n && hgt == o.hgt && w == o.w &&
+               off_image_stride == o.off_image_stride && hmp_plane_stride == o.hmp_plane_stride &&
+               hmp_pixel_stride == o.hmp_pixel_stride && off_plane_stride == o.off_plane_stride &&
+               off_pixel_stride == o.off_pixel_stride && n == o.n && hgt == o.hgt && w == o.w &&
                stride == o.stride && mode == o.mode && flip == o.flip &&
                tables_version == o.tables_version && buffers_version == o.buffers_version;
     }
@@ -127,7 +130,11 @@ struct ResultSlot {
     DevBuf<uint32_t> cand_count;        // K1 pass 1 -> pass 2 hand-over; zero between calls
     DevBuf<uint64_t> cand_keys;
     DevBuf<uint8_t> tile_flag;          // fused K1 scratch: one flag per work block, zero between calls
-    DevBuf<int32_t> tile_list;          // [blocks] work list + the active-block counter at the end
+    // the active-block counter, 3 spare ints, then the [blocks] int4 work list: the counter keeps its
+    // place whatever the geometry of the call, so the select pass that zeroes it leaves it zero for
+    // the next call even when that call lists a different number of blocks
+    DevBuf<int32_t> tile_list;
+    DevBuf<float> nhwc_heat;            // channels-last calls: the scan's flip-fused planar heat maps [n][C][h][w]
     DevBuf<float> limbs;                // K2 output
     GroupScratch group;
     cudaStream_t work = nullptr;        // high priority: K2 -> K3 of every call, the whole chain on the device path
@@ -199,10 +206,8 @@ struct og_handle {
     uint8_t reserved_cache[OG_MAX_LIMBS];
 
     bool timing;
-    struct Plan {                // og_plan_features: the arguments of a repeated device-path decode
-        const void *hmp, *off;
-        int dtype;
-        int64_t hmp_is, off_is;
+    struct Plan {                // og_plan_features_strided: the arguments of a repeated device-path decode
+        MapView hmp, off;        // validated at plan time
         int n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test;
         uint64_t tables_version;
     };
@@ -374,7 +379,9 @@ int run_k3(og_handle *h, GroupScratch &gs, int i0, const float *limbs, bool prep
                         &h->launches);
 }
 
-inline MapView dense_f32(const float *p, size_t per_image) { return MapView{p, OG_DTYPE_F32, per_image}; }
+inline MapView dense_f32(const float *p, size_t per_image, size_t hw) {
+    return MapView::planar(p, OG_DTYPE_F32, per_image, hw);
+}
 inline size_t elem_size(int dtype) { return dtype == OG_DTYPE_F32 ? 4 : 2; }
 inline MapView shift_images(MapView v, size_t images) {
     v.ptr = static_cast<const char *>(v.ptr) + images * v.image_stride * elem_size(v.dtype);
@@ -437,8 +444,10 @@ int begin_call(og_handle *h, ResultSlot *slot, const K1Fused *fused, int n, int 
             const uint8_t *fb = slot->tile_flag.ptr;
             const int32_t *lb = slot->tile_list.ptr;
             OG_TRY(ensure_tracked(slot->tile_flag, flag_bytes, slot));
-            OG_TRY(ensure_tracked(slot->tile_list, tiles + 1, slot));
+            OG_TRY(ensure_tracked(slot->tile_list, tiles + 4, slot));
             fresh_scratch = fresh_scratch || slot->tile_flag.ptr != fb || slot->tile_list.ptr != lb;
+            if (fused->hmp.is_channels_last())
+                OG_TRY(ensure_tracked(slot->nhwc_heat, (size_t)n * c.n_keypoints * fused->h * fused->w, slot));
         }
     }
     if (fresh_scratch) {
@@ -544,15 +553,14 @@ int decode_range(og_handle *h, ResultSlot *slot, int chunk, int i0, int cn, cons
     if (timed) OG_TRY(mark(h, slot, 1, k1s));
     int32_t *n_active = nullptr;
     if (fused) {
-        size_t flag_bytes = 0, tiles = 0;
-        fused_scratch(n, c.n_keypoints, fused->h, fused->w, fused->scale, &flag_bytes, &tiles);
-        n_active = slot->tile_list.ptr + tiles;
+        n_active = slot->tile_list.ptr;
         // the mirrored copy of image i sits n images behind it: shifting the base keeps that offset
         OG_TRY(launch_fused_candidates(shift_images(fused->hmp, i0), h->ft, cn, n,
                                        c.n_keypoints, fused->h, fused->w, fused->scale, fused->cubic,
                                        fused->flip, c.thre_hmp, cand_count, cand_keys, slot->tile_flag.ptr,
-                                       slot->tile_list.ptr, n_active, h->sm_count, !chain, k1s,
-                                       &h->launches));
+                                       slot->tile_list.ptr + 4, n_active,
+                                       slot->nhwc_heat.ptr ? slot->nhwc_heat.ptr + plane0 * fused->h * fused->w : nullptr,
+                                       h->sm_count, !chain, k1s, &h->launches));
     } else {
         OG_TRY(launch_nms_candidates(heat + plane0 * HW, planes, hgt, w, c.thre_hmp, cand_count, cand_keys,
                                      k1s, &h->launches));
@@ -648,6 +656,7 @@ int decode_chain(og_handle *h, ResultSlot *slot, const K1Fused &k1, const Offset
         return finish_call(h, slot);
     }
     const GraphKey key = {k1.hmp.ptr, src.maps.ptr, k1.hmp.dtype, k1.hmp.image_stride, src.maps.image_stride,
+                          k1.hmp.plane_stride, k1.hmp.pixel_stride, src.maps.plane_stride, src.maps.pixel_stride,
                           n, k1.h, k1.w, k1.scale, k1.cubic ? 1 : 0, k1.flip ? 1 : 0, slot->emit_coco ? 1 : 0,
                           h->tables_version, slot->buffers_version,
                           extras ? extras->scale_lr.ptr : nullptr, extras ? extras->jitter_lr.ptr : nullptr,
@@ -750,9 +759,9 @@ int decode_features_impl(og_handle *h, ResultSlot *slot, const float *hmp, const
     if (allow_fused && h->fused_enabled && c.thre_hmp > 0.0f &&
         fused_supported(n, c.n_keypoints, hmp_stride, hgt, w)) {
         OG_TRY(check_maps(n, hgt * hmp_stride, w * hmp_stride, c.n_keypoints));
-        K1Fused k1 = {dense_f32(hmp, (size_t)c.n_keypoints * hw), hgt, w, hmp_stride, resize_mode == 1,
+        K1Fused k1 = {dense_f32(hmp, (size_t)c.n_keypoints * hw, hw), hgt, w, hmp_stride, resize_mode == 1,
                       flip_test != 0};
-        OffsetSource src = {dense_f32(off, (size_t)2 * c.n_limbs * hw), hgt, w, off_stride,
+        OffsetSource src = {dense_f32(off, (size_t)2 * c.n_limbs * hw, hw), hgt, w, off_stride,
                             flip_test ? 1 : 0, n};
         return decode_chain(h, slot, k1, src, n, hgt * hmp_stride, w * hmp_stride, s);
     }
@@ -987,6 +996,7 @@ int og_destroy(og_handle *h) {
         sl.cand_keys.release();
         sl.tile_flag.release();
         sl.tile_list.release();
+        sl.nhwc_heat.release();
         sl.limbs.release();
         sl.redo_lr.release();
         sl.redo_hr.release();
@@ -1220,8 +1230,8 @@ int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float
     const size_t hw = (size_t)hgt * w;
     const int H = hgt * hmp_stride, W = w * hmp_stride;
     OG_TRY(check_maps(n, H, W, c.n_keypoints));
-    K1Fused k1 = {dense_f32(hmp_dev, (size_t)c.n_keypoints * hw), hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
-    OffsetSource src = {dense_f32(off_dev, (size_t)2 * c.n_limbs * hw), hgt, w, off_stride, flip_test ? 1 : 0, n};
+    K1Fused k1 = {dense_f32(hmp_dev, (size_t)c.n_keypoints * hw, hw), hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
+    OffsetSource src = {dense_f32(off_dev, (size_t)2 * c.n_limbs * hw, hw), hgt, w, off_stride, flip_test ? 1 : 0, n};
     LimbExtras ex = {};
     ex.vector_nd = cat_flip_offs ? 4 : 2;
     ex.use_jitter = use_jitter ? 1 : 0;
@@ -1234,23 +1244,44 @@ int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float
 
 namespace {
 
-// og_decode_features_dev_ex behind its argument checks (also the body of a plan launch)
-int decode_dev_views(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
-                     int64_t hmp_image_stride, int64_t off_image_stride, int n, int hgt, int w,
-                     int hmp_stride, int off_stride, int resize_mode, int flip_test, cudaStream_t s) {
+// The view of one map from its element strides in (image, channel, row, column) order: planar
+// (s_n, h * w, w, 1) or channels-last (s_n, 1, w * p, p) with p >= channels; s_n must cover an image
+// unless the buffer holds a single one.  A layout that is both is planar.  Anything else is refused
+// here, before any launch.
+int map_view(const char *name, const void *ptr, int dtype, const int64_t st[4], int channels, int images, int hgt,
+             int w, MapView *out) {
+    OG_REQUIRE(st != nullptr, "%s: null stride array", name);
+    const int64_t hw = (int64_t)hgt * w;
+    if (st[3] == 1 && st[2] == w && st[1] == hw) {
+        OG_REQUIRE(images <= 1 || st[0] >= channels * hw,
+                   "%s: image stride %lld is smaller than one planar image (%lld elements)", name,
+                   (long long)st[0], (long long)(channels * hw));
+        *out = MapView::planar(ptr, dtype, (size_t)std::max<int64_t>(st[0], channels * hw), (size_t)hw);
+        return OG_OK;
+    }
+    const int64_t p = st[3];
+    OG_REQUIRE(st[1] == 1 && p >= channels && st[2] == w * p,
+               "%s: strides (%lld, %lld, %lld, %lld) are neither planar (s_n, %lld, %d, 1) nor channels-last "
+               "(s_n, 1, %d * p, p) with p >= %d channels", name, (long long)st[0], (long long)st[1],
+               (long long)st[2], (long long)st[3], (long long)hw, w, w, channels);
+    OG_REQUIRE(images <= 1 || st[0] >= hw * p,
+               "%s: image stride %lld is smaller than one channels-last image (%lld elements)", name,
+               (long long)st[0], (long long)(hw * p));
+    *out = MapView::channels_last(ptr, dtype, (size_t)std::max<int64_t>(st[0], hw * p), (size_t)p);
+    return OG_OK;
+}
+
+// og_decode_features_dev_strided behind its argument checks (also the body of a plan launch)
+int decode_dev_views(og_handle *h, const MapView &hv, const MapView &ov, int n, int hgt, int w, int hmp_stride,
+                     int off_stride, int resize_mode, int flip_test, cudaStream_t s) {
     const og_config &c = h->cfg;
     const size_t hw = (size_t)hgt * w;
     const size_t hmp_img = (size_t)c.n_keypoints * hw, off_img = (size_t)2 * c.n_limbs * hw;
-    OG_REQUIRE(hmp_image_stride == 0 || (size_t)hmp_image_stride >= hmp_img,
-               "hmp_image_stride %lld is smaller than one image (%zu elements)", (long long)hmp_image_stride, hmp_img);
-    OG_REQUIRE(off_image_stride == 0 || (size_t)off_image_stride >= off_img,
-               "off_image_stride %lld is smaller than one image (%zu elements)", (long long)off_image_stride, off_img);
-    MapView hv = {hmp_dev, dtype, hmp_image_stride ? (size_t)hmp_image_stride : hmp_img};
-    MapView ov = {off_dev, dtype, off_image_stride ? (size_t)off_image_stride : off_img};
-    if (dtype == OG_DTYPE_F32 && hv.image_stride == hmp_img && ov.image_stride == off_img) {
+    if (hv.dtype == OG_DTYPE_F32 && !hv.is_channels_last() && !ov.is_channels_last() && hv.image_stride == hmp_img &&
+        ov.image_stride == off_img) {
         ResultSlot *slot = nullptr;
         OG_TRY(acquire_slot(h, nullptr, &slot));
-        return decode_features_impl(h, slot, static_cast<const float *>(hmp_dev), static_cast<const float *>(off_dev),
+        return decode_features_impl(h, slot, static_cast<const float *>(hv.ptr), static_cast<const float *>(ov.ptr),
                                     n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, s, true);
     }
     if (!(h->fused_enabled && c.thre_hmp > 0.0f && fused_supported(n, c.n_keypoints, hmp_stride, hgt, w))) {
@@ -1267,7 +1298,51 @@ int decode_dev_views(og_handle *h, const void *hmp_dev, const void *off_dev, int
     return decode_chain(h, slot, k1, src, n, H, W, s);
 }
 
+int check_dtype(int dtype) {
+    OG_REQUIRE(dtype == OG_DTYPE_F32 || dtype == OG_DTYPE_BF16 || dtype == OG_DTYPE_F16,
+               "dtype must be OG_DTYPE_F32, OG_DTYPE_BF16 or OG_DTYPE_F16");
+    return OG_OK;
+}
+
+// the element strides of og_decode_features_dev_ex's planar views (image stride 0 = dense)
+int planar_strides(const char *name, int64_t image_stride, int channels, int hgt, int w, int64_t out[4]) {
+    const int64_t hw = (int64_t)hgt * w;
+    OG_REQUIRE(image_stride == 0 || image_stride >= channels * hw,
+               "%s %lld is smaller than one image (%lld elements)", name, (long long)image_stride,
+               (long long)(channels * hw));
+    out[0] = image_stride ? image_stride : channels * hw;
+    out[1] = hw;
+    out[2] = w;
+    out[3] = 1;
+    return OG_OK;
+}
+
+// validated views of both maps
+int feature_views(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype, const int64_t *hmp_st,
+                  const int64_t *off_st, int n, int hgt, int w, int flip_test, MapView *hv, MapView *ov) {
+    const int images = flip_test ? 2 * n : n;
+    OG_TRY(map_view("hmp_elem_strides", hmp_dev, dtype, hmp_st, h->cfg.n_keypoints, images, hgt, w, hv));
+    OG_TRY(map_view("off_elem_strides", off_dev, dtype, off_st, 2 * h->cfg.n_limbs, images, hgt, w, ov));
+    return OG_OK;
+}
+
 }  // namespace
+
+int og_decode_features_dev_strided(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
+                                   const int64_t hmp_elem_strides[4], const int64_t off_elem_strides[4], int n,
+                                   int hgt, int w, int hmp_stride, int off_stride, int resize_mode, int flip_test,
+                                   const int32_t *kp_flip, const int32_t *limb_flip,
+                                   const int32_t *limb_reserve, int n_reserve, void *stream) {
+    OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_dev_strided: null pointer");
+    OG_TRY(check_dtype(dtype));
+    OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
+                              limb_flip, limb_reserve, n_reserve));
+    MapView hv, ov;
+    OG_TRY(feature_views(h, hmp_dev, off_dev, dtype, hmp_elem_strides, off_elem_strides, n, hgt, w, flip_test, &hv,
+                         &ov));
+    return decode_dev_views(h, hv, ov, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test,
+                            static_cast<cudaStream_t>(stream));
+}
 
 int og_decode_features_dev_ex(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
                               int64_t hmp_image_stride, int64_t off_image_stride, int n, int hgt,
@@ -1275,19 +1350,22 @@ int og_decode_features_dev_ex(og_handle *h, const void *hmp_dev, const void *off
                               const int32_t *kp_flip, const int32_t *limb_flip,
                               const int32_t *limb_reserve, int n_reserve, void *stream) {
     OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_dev_ex: null pointer");
-    OG_REQUIRE(dtype == OG_DTYPE_F32 || dtype == OG_DTYPE_BF16 || dtype == OG_DTYPE_F16,
-               "dtype must be OG_DTYPE_F32, OG_DTYPE_BF16 or OG_DTYPE_F16");
+    OG_TRY(check_dtype(dtype));
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
                               limb_flip, limb_reserve, n_reserve));
-    return decode_dev_views(h, hmp_dev, off_dev, dtype, hmp_image_stride, off_image_stride, n, hgt, w, hmp_stride,
-                            off_stride, resize_mode, flip_test, static_cast<cudaStream_t>(stream));
+    int64_t hs[4], os[4];
+    OG_TRY(planar_strides("hmp_image_stride", hmp_image_stride, h->cfg.n_keypoints, hgt, w, hs));
+    OG_TRY(planar_strides("off_image_stride", off_image_stride, 2 * h->cfg.n_limbs, hgt, w, os));
+    return og_decode_features_dev_strided(h, hmp_dev, off_dev, dtype, hs, os, n, hgt, w, hmp_stride, off_stride,
+                                          resize_mode, flip_test, kp_flip, limb_flip, limb_reserve, n_reserve,
+                                          stream);
 }
 
-int og_plan_features(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
-                     int64_t hmp_image_stride, int64_t off_image_stride, int n, int hgt, int w,
-                     int hmp_stride, int off_stride, int resize_mode, int flip_test,
-                     const int32_t *kp_flip, const int32_t *limb_flip, const int32_t *limb_reserve,
-                     int n_reserve, int32_t *plan_id) {
+int og_plan_features_strided(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
+                             const int64_t hmp_elem_strides[4], const int64_t off_elem_strides[4], int n, int hgt,
+                             int w, int hmp_stride, int off_stride, int resize_mode, int flip_test,
+                             const int32_t *kp_flip, const int32_t *limb_flip, const int32_t *limb_reserve,
+                             int n_reserve, int32_t *plan_id) {
     OG_REQUIRE(h && plan_id, "og_plan_features: null pointer");
     *plan_id = -1;
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
@@ -1303,12 +1381,29 @@ int og_plan_features(og_handle *h, const void *hmp_dev, const void *off_dev, int
         h->cap_plans = cap;
     }
     OG_REQUIRE(hmp_dev && off_dev && n > 0, "og_plan_features: null pointer or empty batch");
-    OG_REQUIRE(dtype == OG_DTYPE_F32 || dtype == OG_DTYPE_BF16 || dtype == OG_DTYPE_F16,
-               "dtype must be OG_DTYPE_F32, OG_DTYPE_BF16 or OG_DTYPE_F16");
-    h->plans[h->n_plans] = og_handle::Plan{hmp_dev, off_dev, dtype, hmp_image_stride, off_image_stride, n, hgt, w,
-                                           hmp_stride, off_stride, resize_mode, flip_test, h->tables_version};
+    OG_TRY(check_dtype(dtype));
+    MapView hv, ov;
+    OG_TRY(feature_views(h, hmp_dev, off_dev, dtype, hmp_elem_strides, off_elem_strides, n, hgt, w, flip_test, &hv,
+                         &ov));
+    h->plans[h->n_plans] = og_handle::Plan{hv, ov, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test,
+                                           h->tables_version};
     *plan_id = h->n_plans++;
     return OG_OK;
+}
+
+int og_plan_features(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,
+                     int64_t hmp_image_stride, int64_t off_image_stride, int n, int hgt, int w,
+                     int hmp_stride, int off_stride, int resize_mode, int flip_test,
+                     const int32_t *kp_flip, const int32_t *limb_flip, const int32_t *limb_reserve,
+                     int n_reserve, int32_t *plan_id) {
+    OG_REQUIRE(h && plan_id, "og_plan_features: null pointer");
+    *plan_id = -1;
+    OG_TRY(check_maps(n, hgt, w, h->cfg.n_keypoints));
+    int64_t hs[4], os[4];
+    OG_TRY(planar_strides("hmp_image_stride", hmp_image_stride, h->cfg.n_keypoints, hgt, w, hs));
+    OG_TRY(planar_strides("off_image_stride", off_image_stride, 2 * h->cfg.n_limbs, hgt, w, os));
+    return og_plan_features_strided(h, hmp_dev, off_dev, dtype, hs, os, n, hgt, w, hmp_stride, off_stride,
+                                    resize_mode, flip_test, kp_flip, limb_flip, limb_reserve, n_reserve, plan_id);
 }
 
 int og_plan_launch(og_handle *h, int32_t plan_id, void *stream) {
@@ -1317,8 +1412,8 @@ int og_plan_launch(og_handle *h, int32_t plan_id, void *stream) {
     OG_REQUIRE(!p.flip_test || p.tables_version == h->tables_version,
                "og_plan_launch: the flip tables changed since plan %d was made", plan_id);
     OG_TRY(check_device(h));
-    return decode_dev_views(h, p.hmp, p.off, p.dtype, p.hmp_is, p.off_is, p.n, p.hgt, p.w, p.hmp_stride, p.off_stride,
-                            p.resize_mode, p.flip_test, static_cast<cudaStream_t>(stream));
+    return decode_dev_views(h, p.hmp, p.off, p.n, p.hgt, p.w, p.hmp_stride, p.off_stride, p.resize_mode,
+                            p.flip_test, static_cast<cudaStream_t>(stream));
 }
 
 int og_decode_features_host(og_handle *h, const float *hmp_host, const float *off_host, int n,
@@ -1390,8 +1485,8 @@ int og_decode_features_host(og_handle *h, const float *hmp_host, const float *of
     }
     const int H = hgt * hmp_stride, W = w * hmp_stride;
     OG_TRY(check_maps(n, H, W, c.n_keypoints));
-    K1Fused k1 = {dense_f32(slot->in_hmp.ptr, hmp_img), hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
-    OffsetSource src = {dense_f32(off_src, off_img), hgt, w, off_stride, flip_test ? 1 : 0, n};
+    K1Fused k1 = {dense_f32(slot->in_hmp.ptr, hmp_img, hw), hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
+    OffsetSource src = {dense_f32(off_src, off_img, hw), hgt, w, off_stride, flip_test ? 1 : 0, n};
     OG_TRY(begin_call(h, slot, &k1, n, H, W, s));
     // Image ranges: only the kernels of the LAST range run after the last byte has arrived, so
     // that range is kept small (n / 16, at least 4 images); the others share the rest evenly.

@@ -120,11 +120,29 @@ int launch_select_topk(const float *heat, int planes, int h, int w, float thre, 
 // Element types: float32 (what the reference decodes, factory.py:59), or bfloat16 / float16
 // straight from a reduced-precision head (SURVEY 8f-4).  Such a value widens exactly to float32, so everything after the
 // load is the float32 path bit for bit.  Images may be `image_stride` elements apart (channel
-// slices of one packed [N, 55, h, w] network output); the planes of an image are contiguous.
+// slices of one packed [N, 55, h, w] network output).  Cell (y, x) of channel ch of image i is
+// element i * image_stride + ch * plane_stride + (y * w + x) * pixel_stride: planar maps have
+// plane_stride = h * w, pixel_stride = 1; channels-last (NHWC) maps plane_stride = 1 and
+// pixel_stride = the channel count of the whole packed tensor.  Built through the factories only,
+// so no view can leave a stride unset.
 struct MapView {
-    const void *ptr;
-    int dtype;                      // OG_DTYPE_F32 / OG_DTYPE_BF16 / OG_DTYPE_F16
-    size_t image_stride;            // elements between consecutive images
+    const void *ptr = nullptr;
+    int dtype = OG_DTYPE_F32;       // OG_DTYPE_F32 / OG_DTYPE_BF16 / OG_DTYPE_F16
+    size_t image_stride = 0;        // elements between consecutive images
+    size_t plane_stride = 0;        // elements between consecutive channels
+    size_t pixel_stride = 1;        // elements between consecutive cells of a row
+    MapView() = default;
+    static MapView planar(const void *p, int dtype, size_t image_stride, size_t hw) {
+        return MapView(p, dtype, image_stride, hw, 1);
+    }
+    static MapView channels_last(const void *p, int dtype, size_t image_stride, size_t pixel_stride) {
+        return MapView(p, dtype, image_stride, 1, pixel_stride);
+    }
+    bool is_channels_last() const { return pixel_stride != 1; }
+
+private:
+    MapView(const void *p, int dt, size_t is, size_t ps, size_t xs)
+        : ptr(p), dtype(dt), image_stride(is), plane_stride(ps), pixel_stride(xs) {}
 };
 #ifdef __CUDACC__
 __device__ __forceinline__ float load_cell(const float *p) { return __ldg(p); }
@@ -148,7 +166,7 @@ struct FlipTablesDev {
 };
 
 struct OffsetSource {
-    MapView maps;                   // [n or 2n][2L][h][w]
+    MapView maps;                   // [n or 2n][2L][h][w], planar or channels-last
     int h, w, scale;                // network resolution and the x scale to decode resolution
     int flip, n;                    // flip: maps = n originals then n mirrored copies
 };
@@ -208,16 +226,18 @@ void fused_scratch(int n, int c, int h, int w, int scale, size_t *flag_bytes, si
 // `clear_first`: zero the candidate counters / the active-block counter with memsets before the
 // kernels (a caller whose select pass runs on ANOTHER stream); otherwise they must be zero on
 // entry (launch_select_topk leaves them so).
+// Channels-last heat maps: the activity scan transposes them, flip-fused, into `nhwc_heat`
+// (dense float32 [n][c][h][w], ignored for planar maps), and the block kernel reads that.
 int launch_fused_candidates(const MapView &hmp, const FlipTablesDev &flips, int n, int n_total, int c, int h, int w,
                             int scale, bool cubic, bool flip, float thre, uint32_t *cand_count,
                             uint64_t *cand_keys, uint8_t *block_flag, int32_t *block_list,
-                            int32_t *n_active, int sm_count, bool clear_first, cudaStream_t s,
-                            int64_t *launches);
+                            int32_t *n_active, float *nhwc_heat, int sm_count, bool clear_first,
+                            cudaStream_t s, int64_t *launches);
 
-// Network-resolution planes plane_list[0 .. count) (plane = image * C + channel) of `hmp` as dense
-// float32, averaged with their mirrored partners when `flip` (factory.py:101-106): the input of the
-// exact per-plane redo of a fused decode.  `n` = images of the call (the mirrored copy of image i
-// is image n + i).
+// Network-resolution planes plane_list[0 .. count) (plane = image * C + channel) of `hmp` (either
+// layout) as dense float32, averaged with their mirrored partners when `flip` (factory.py:101-106):
+// the input of the exact per-plane redo of a fused decode.  `n` = images of the call (the mirrored
+// copy of image i is image n + i).
 int launch_fuse_planes(const MapView &hmp, const FlipTablesDev &flips, int n, int c, int h, int w, bool flip,
                        const int32_t *plane_list, int count, float *out, cudaStream_t s);
 

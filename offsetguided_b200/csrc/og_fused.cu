@@ -167,6 +167,67 @@ amax_scan_kernel(const T *__restrict__ hmp, size_t img_stride, const FlipTablesD
     }
 }
 
+// ---- pass A for channels-last maps: transposing activity scan ------------------------
+// Cell (y, x) of channel c is at (y * w + x) * P + c (P >= C: the channel count of the packed
+// tensor), so a plane's cells are P elements apart and a block kernel gathering them would touch
+// a 32-byte sector per cell.  This pass is the only one over the channels-last heat channels: it
+// reads each pixel's C channels (with flip-test also the mirrored image's pixel w - 1 - x, channel
+// kp[c]), writes the fused values as dense float32 planes `out` [n][C][h][w] for the block kernel,
+// and flags exactly the blocks amax_scan_kernel would flag on those planes.
+// One CTA per (image, 8-row band, 32-pixel column group).  A row's 32 x C values are loaded with
+// consecutive threads on consecutive channels of consecutive pixels (coalesced along the pixel run),
+// staged in shared memory, and written as 32-cell runs of each plane.
+constexpr int kNhwcPixels = 32;
+constexpr int kNhwcThreads = 256;
+
+template <typename T, bool kFlip>
+__global__ void __launch_bounds__(kNhwcThreads)
+amax_scan_nhwc_kernel(const T *__restrict__ hmp, size_t img_stride, size_t pix_stride, const FlipTablesDev ft,
+                      int N, int C, int h, int w, int bw_shift, int halo, float limit,
+                      uint8_t *__restrict__ block_flag, float *__restrict__ out) {
+    __shared__ float s_row[OG_MAX_KEYPOINTS][kNhwcPixels + 1];
+    const int gxs = (w + kNhwcPixels - 1) / kNhwcPixels, bands = (h + kBlockCellsH - 1) / kBlockCellsH;
+    const unsigned cta = blockIdx.x;
+    const int gx = (int)(cta % (unsigned)gxs);
+    const int band = (int)((cta / (unsigned)gxs) % (unsigned)bands);
+    const int n = (int)(cta / ((unsigned)gxs * (unsigned)bands));
+    const int x0 = gx * kNhwcPixels, y0 = band * kBlockCellsH;
+    const int px_n = min(kNhwcPixels, w - x0), y_end = min(y0 + kBlockCellsH, h);
+    const int block_w = 1 << bw_shift;
+    const int bxs = (w + block_w - 1) >> bw_shift, bys = (h + kBlockCellsH - 1) / kBlockCellsH;
+    const size_t hw = (size_t)h * w;
+    const T *a = hmp + (size_t)n * img_stride;
+    const T *b = kFlip ? hmp + (size_t)(N + n) * img_stride : nullptr;
+    const int cells = px_n * C;
+    for (int y = y0; y < y_end; ++y) {
+        for (int i = threadIdx.x; i < cells; i += kNhwcThreads) {
+            const int px = i / C, c = i - px * C;
+            const int x = x0 + px;
+            float v = load_cell(a + ((size_t)y * w + x) * pix_stride + c);
+            if (kFlip)                       // (orig + flip_W(flipped)[kp_flip]) / 2, factory.py:101-106
+                v = __fmul_rn(__fadd_rn(v, load_cell(b + ((size_t)y * w + (w - 1 - x)) * pix_stride + ft.kp[c])), 0.5f);
+            s_row[c][px] = v;
+        }
+        __syncthreads();
+        for (int j = threadIdx.x; j < C * kNhwcPixels; j += kNhwcThreads) {
+            const int c = j / kNhwcPixels, px = j - c * kNhwcPixels;
+            if (px >= px_n) continue;
+            const int x = x0 + px;
+            const float v = s_row[c][px];
+            const int plane = n * C + c;
+            out[(size_t)plane * hw + (size_t)y * w + x] = v;
+            if (!(fabsf(v) < limit)) {       // NaN is not below: stays active
+                uint8_t *flags = block_flag + (size_t)plane * bys * bxs;
+                const int bx_lo = max(x - halo, 0) >> bw_shift, bx_hi = min((x + halo) >> bw_shift, bxs - 1);
+                const int by_lo = max(y - halo, 0) / kBlockCellsH, by_hi = min((y + halo) / kBlockCellsH, bys - 1);
+                for (int by = by_lo; by <= by_hi; ++by)
+                    for (int bx = bx_lo; bx <= bx_hi; ++bx) flags[by * bxs + bx] = 1;
+            }
+        }
+        __syncthreads();
+    }
+}
+
 // ---- pass B: work list -----------------------------------------------------------
 // Compacts the flagged blocks and clears the flags for the next call.
 // entry = {plane (image * C + channel), image, block row << 16 | block column,
@@ -481,22 +542,51 @@ void fused_scratch(int n, int c, int h, int w, int scale, size_t *flag_bytes, si
 }
 
 namespace {
+// the activity scan's parameters: log2 of the block width in cells, the tap halo and the cell limit
+inline int scan_bw_shift(int scale) { return scale == 2 ? 4 : (scale == 4 ? 3 : 2); }
+inline int scan_halo(bool cubic) { return cubic ? 2 : 1; }
+inline float scan_limit(float thre, bool cubic) { return thre / (cubic ? 1.95f : 1.001f); }
+
+template <typename T>
+int launch_scan_nhwc_t(const T *hmp, size_t img_stride, size_t pix_stride, const FlipTablesDev &kp_flip_dev, int n,
+                       int n_total, int c, int h, int w, int scale, bool cubic, bool flip, float thre,
+                       uint8_t *block_flag, float *out, cudaStream_t s) {
+    const long long ctas = (long long)n * ((w + kNhwcPixels - 1) / kNhwcPixels) *
+                           ((h + kBlockCellsH - 1) / kBlockCellsH);
+    if (ctas > 0x7fffffffLL) {
+        set_error("fused K1: %lld scan CTAs of channels-last maps exceed one launch", ctas);
+        return OG_ERR_UNSUPPORTED;
+    }
+#define OG_SCAN_NHWC(FLIP)                                                                                      \
+    (prefer_chain_carveout<amax_scan_nhwc_kernel<T, FLIP>>(),                                                    \
+     amax_scan_nhwc_kernel<T, FLIP><<<(unsigned)ctas, kNhwcThreads, 0, s>>>(                                     \
+         hmp, img_stride, pix_stride, kp_flip_dev, n_total, c, h, w, scan_bw_shift(scale), scan_halo(cubic),     \
+         scan_limit(thre, cubic), block_flag, out))
+    if (flip) OG_SCAN_NHWC(true); else OG_SCAN_NHWC(false);
+#undef OG_SCAN_NHWC
+    OG_CUDA_TRY(cudaGetLastError());
+    return OG_OK;
+}
+
+// `scan`: run the activity scan over `hmp`; false when the transposing scan already flagged the
+// blocks and wrote `hmp` (its dense float32 output)
 template <typename T>
 int launch_fused_t(const T *hmp, size_t img_stride, const FlipTablesDev &kp_flip_dev, int n, int n_total,
                    int c, int h, int w, int scale, bool cubic, bool flip, float thre,
                    uint32_t *cand_count, uint64_t *cand_keys, uint8_t *block_flag, int32_t *block_list,
-                   int32_t *n_active, int sm_count, bool clear_first, cudaStream_t s, int64_t *launches) {
+                   int32_t *n_active, int sm_count, bool clear_first, bool scan, cudaStream_t s,
+                   int64_t *launches) {
     if (clear_first) {
         OG_CUDA_TRY(cudaMemsetAsync(cand_count, 0, sizeof(uint32_t) * (size_t)n * c, s));
         OG_CUDA_TRY(cudaMemsetAsync(n_active, 0, sizeof(int32_t), s));
     }
 
     const int sxs = (w + kSub - 1) / kSub, bands = (h + 2 * kSub - 1) / (2 * kSub);
-    const int per_plane = bands * sxs, planes = n * c;
-    const int planes_per_launch = std::max(1, (int)std::min<long long>(planes, 0x7fffffffLL / per_plane - 1));
-    const int block_w = 32 / scale, halo = cubic ? 2 : 1;
-    const int bw_shift = scale == 2 ? 4 : (scale == 4 ? 3 : 2);
-    const float limit = thre / (cubic ? 1.95f : 1.001f);
+    const int per_plane = bands * sxs, planes = scan ? n * c : 0;
+    const int planes_per_launch = std::max(1, (int)std::min<long long>(n * c, 0x7fffffffLL / per_plane - 1));
+    const int block_w = 32 / scale, halo = scan_halo(cubic);
+    const int bw_shift = scan_bw_shift(scale);
+    const float limit = scan_limit(thre, cubic);
     // vector loads need whole 4-cell groups and rows aligned to the 4-cell load size (also the
     // rows of the mirrored read and of every image)
     const size_t vec_bytes = 4 * sizeof(T);
@@ -541,24 +631,46 @@ int launch_fused_t(const T *hmp, size_t img_stride, const FlipTablesDev &kp_flip
 int launch_fused_candidates(const MapView &hmp, const FlipTablesDev &kp_flip_dev, int n, int n_total, int c,
                             int h, int w, int scale, bool cubic, bool flip, float thre,
                             uint32_t *cand_count, uint64_t *cand_keys, uint8_t *block_flag,
-                            int32_t *block_list, int32_t *n_active, int sm_count, bool clear_first,
-                            cudaStream_t s, int64_t *launches) {
+                            int32_t *block_list, int32_t *n_active, float *nhwc_heat, int sm_count,
+                            bool clear_first, cudaStream_t s, int64_t *launches) {
     if (n == 0) return OG_OK;
     if (!fused_supported(n, c, scale, h, w)) {
         set_error("fused K1: scale %d / %d x %d maps are outside the supported range", scale, h, w);
         return OG_ERR_UNSUPPORTED;
     }
+    if (hmp.is_channels_last()) {
+        // the transposing scan replaces the planar one; the block kernel then runs on its dense
+        // float32, already flip-fused output (no mirrored image left to read)
+        if (clear_first) {          // before the scan: the counters of an earlier range may still be read
+            OG_CUDA_TRY(cudaMemsetAsync(cand_count, 0, sizeof(uint32_t) * (size_t)n * c, s));
+            OG_CUDA_TRY(cudaMemsetAsync(n_active, 0, sizeof(int32_t), s));
+        }
+        int st;
+        if (hmp.dtype == OG_DTYPE_BF16)
+            st = launch_scan_nhwc_t(static_cast<const __nv_bfloat16 *>(hmp.ptr), hmp.image_stride, hmp.pixel_stride,
+                                    kp_flip_dev, n, n_total, c, h, w, scale, cubic, flip, thre, block_flag, nhwc_heat, s);
+        else if (hmp.dtype == OG_DTYPE_F16)
+            st = launch_scan_nhwc_t(static_cast<const __half *>(hmp.ptr), hmp.image_stride, hmp.pixel_stride,
+                                    kp_flip_dev, n, n_total, c, h, w, scale, cubic, flip, thre, block_flag, nhwc_heat, s);
+        else
+            st = launch_scan_nhwc_t(static_cast<const float *>(hmp.ptr), hmp.image_stride, hmp.pixel_stride,
+                                    kp_flip_dev, n, n_total, c, h, w, scale, cubic, flip, thre, block_flag, nhwc_heat, s);
+        OG_TRY(st);
+        return launch_fused_t(static_cast<const float *>(nhwc_heat), (size_t)c * h * w, kp_flip_dev, n, n, c, h, w,
+                              scale, cubic, false, thre, cand_count, cand_keys, block_flag, block_list, n_active,
+                              sm_count, false, false, s, launches);
+    }
     if (hmp.dtype == OG_DTYPE_BF16)
         return launch_fused_t(static_cast<const __nv_bfloat16 *>(hmp.ptr), hmp.image_stride, kp_flip_dev, n,
                               n_total, c, h, w, scale, cubic, flip, thre, cand_count, cand_keys, block_flag,
-                              block_list, n_active, sm_count, clear_first, s, launches);
+                              block_list, n_active, sm_count, clear_first, true, s, launches);
     if (hmp.dtype == OG_DTYPE_F16)
         return launch_fused_t(static_cast<const __half *>(hmp.ptr), hmp.image_stride, kp_flip_dev, n,
                               n_total, c, h, w, scale, cubic, flip, thre, cand_count, cand_keys, block_flag,
-                              block_list, n_active, sm_count, clear_first, s, launches);
+                              block_list, n_active, sm_count, clear_first, true, s, launches);
     return launch_fused_t(static_cast<const float *>(hmp.ptr), hmp.image_stride, kp_flip_dev, n, n_total, c,
                           h, w, scale, cubic, flip, thre, cand_count, cand_keys, block_flag, block_list,
-                          n_active, sm_count, clear_first, s, launches);
+                          n_active, sm_count, clear_first, true, s, launches);
 }
 
 // single network-resolution planes as dense float32, flip-fused (the exact per-plane redo of a
@@ -566,20 +678,21 @@ int launch_fused_candidates(const MapView &hmp, const FlipTablesDev &kp_flip_dev
 // overflowed)
 namespace {
 template <typename T>
-__global__ void fuse_planes_kernel(const T *__restrict__ hmp, size_t img_stride, const FlipTablesDev ft, int n,
+__global__ void fuse_planes_kernel(const T *__restrict__ hmp, size_t img_stride, size_t plane_stride,
+                                   size_t pix_stride, const FlipTablesDev ft, int n,
                                    int C, int h, int w, int flip, const int32_t *__restrict__ plane_list,
                                    float *__restrict__ out) {
     const int plane = plane_list[blockIdx.y];
     const int img = plane / C, c = plane - img * C;
     const size_t hw = (size_t)h * w;
-    const T *a = hmp + (size_t)img * img_stride + (size_t)c * hw;
-    const T *b = flip ? hmp + (size_t)(n + img) * img_stride + (size_t)ft.kp[c] * hw : nullptr;
+    const T *a = hmp + (size_t)img * img_stride + (size_t)c * plane_stride;
+    const T *b = flip ? hmp + (size_t)(n + img) * img_stride + (size_t)ft.kp[c] * plane_stride : nullptr;
     float *o = out + (size_t)blockIdx.y * hw;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < hw; i += (size_t)gridDim.x * blockDim.x) {
-        float v = load_cell(a + i);
+        float v = load_cell(a + i * pix_stride);
         if (flip) {                          // (orig + flip_W(flipped)[kp_flip]) / 2, factory.py:101-106
             const int y = (int)(i / w), x = (int)(i - (size_t)y * w);
-            v = __fmul_rn(__fadd_rn(v, load_cell(b + (size_t)y * w + (w - 1 - x))), 0.5f);
+            v = __fmul_rn(__fadd_rn(v, load_cell(b + ((size_t)y * w + (w - 1 - x)) * pix_stride)), 0.5f);
         }
         o[i] = v;
     }
@@ -592,11 +705,11 @@ int launch_fuse_planes(const MapView &hmp, const FlipTablesDev &flips, int n, in
     const size_t hw = (size_t)h * w;
     const dim3 grid((unsigned)std::min<size_t>((hw + 255) / 256, 64), (unsigned)count);
     if (hmp.dtype == OG_DTYPE_BF16)
-        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const __nv_bfloat16 *>(hmp.ptr), hmp.image_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
+        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const __nv_bfloat16 *>(hmp.ptr), hmp.image_stride, hmp.plane_stride, hmp.pixel_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
     else if (hmp.dtype == OG_DTYPE_F16)
-        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const __half *>(hmp.ptr), hmp.image_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
+        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const __half *>(hmp.ptr), hmp.image_stride, hmp.plane_stride, hmp.pixel_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
     else
-        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const float *>(hmp.ptr), hmp.image_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
+        fuse_planes_kernel<<<grid, 256, 0, s>>>(static_cast<const float *>(hmp.ptr), hmp.image_stride, hmp.plane_stride, hmp.pixel_stride, flips, n, c, h, w, flip ? 1 : 0, plane_list, out);
     OG_CUDA_TRY(cudaGetLastError());
     return OG_OK;
 }

@@ -37,18 +37,19 @@ __device__ __forceinline__ float norm2(float dx, float dy) {
 // interpolation on the fly (bilinear or bicubic, ATen's taps and accumulation order, og_interp.cuh),
 // optionally fused with the flip-test combination of plane `a` (original image) and plane `b`
 // (mirrored image, read right-to-left) — bit-identical to gathering from the materialised
-// flip_augment + F.interpolate(scale_factor = S) map.
+// flip_augment + F.interpolate(scale_factor = S) map.  Cell (y, x) of a plane is `pixel_stride`
+// elements after cell (y, x - 1): 1 for planar maps, the packed channel count for channels-last.
 enum FlipMode { kFlipNone = 0, kFlipAverage = 1, kFlipPartnerOnly = 2 };
 
 template <typename T>
 __device__ __forceinline__ float sample_lowres(const T *a, const T *b, int mode, bool negate_b, int h, int w,
-                                               int scale, bool cubic, int X, int Y) {
+                                               size_t pixel_stride, int scale, bool cubic, int X, int Y) {
     auto at = [&](int yy, int xx) {
-        if (mode == kFlipNone) return load_cell(a + yy * w + xx);
-        float m = load_cell(b + yy * w + (w - 1 - xx));
+        if (mode == kFlipNone) return load_cell(a + (size_t)(yy * w + xx) * pixel_stride);
+        float m = load_cell(b + (size_t)(yy * w + (w - 1 - xx)) * pixel_stride);
         if (negate_b) m = -m;
         if (mode == kFlipPartnerOnly) return m;
-        return __fmul_rn(__fadd_rn(load_cell(a + yy * w + xx), m), 0.5f);
+        return __fmul_rn(__fadd_rn(load_cell(a + (size_t)(yy * w + xx) * pixel_stride), m), 0.5f);
     };
     if (scale == 1) return at(Y, X);
     const float inv = 1.0f / (float)scale;
@@ -75,17 +76,16 @@ __device__ __forceinline__ float sample_lowres(const T *a, const T *b, int mode,
 template <typename T>
 __device__ __forceinline__ float sample_offset_t(const OffsetSource &src, const FlipTablesDev &ft, int img, int l,
                                                  int comp, bool cat, int X, int Y) {
-    const size_t hw = (size_t)src.h * src.w;
     const T *base = static_cast<const T *>(src.maps.ptr);
     const int c2 = comp & 1;
-    const T *a = base + (size_t)img * src.maps.image_stride + (size_t)(2 * l + c2) * hw;
+    const T *a = base + (size_t)img * src.maps.image_stride + (size_t)(2 * l + c2) * src.maps.plane_stride;
     const bool mirrored = src.flip && !((ft.reserved >> l) & 1ull);
     const T *b = mirrored ? base + (size_t)(src.n + img) * src.maps.image_stride +
-                                (size_t)(2 * (int)ft.limb[l] + c2) * hw
+                                (size_t)(2 * (int)ft.limb[l] + c2) * src.maps.plane_stride
                           : nullptr;
     int mode = kFlipNone;
     if (mirrored) mode = cat ? (comp >= 2 ? kFlipPartnerOnly : kFlipNone) : kFlipAverage;
-    return sample_lowres(a, b, mode, c2 == 0, src.h, src.w, src.scale, false, X, Y);
+    return sample_lowres(a, b, mode, c2 == 0, src.h, src.w, src.maps.pixel_stride, src.scale, false, X, Y);
 }
 
 __device__ __forceinline__ float sample_offset(const OffsetSource &src, const FlipTablesDev &ft, int img, int l,
@@ -103,7 +103,7 @@ __device__ __forceinline__ float sample_head(const HeadSource &hs, const OffsetS
     const size_t hw = (size_t)hs.h * hs.w;
     const float *a = hs.ptr + ((size_t)img * channels + ch) * hw;
     const float *b = src.flip ? hs.ptr + ((size_t)(src.n + img) * channels + partner) * hw : nullptr;
-    return sample_lowres(a, b, src.flip ? kFlipAverage : kFlipNone, negate_partner, hs.h, hs.w, hs.scale,
+    return sample_lowres(a, b, src.flip ? kFlipAverage : kFlipNone, negate_partner, hs.h, hs.w, (size_t)1, hs.scale,
                          hs.cubic != 0, X, Y);
 }
 

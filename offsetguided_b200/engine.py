@@ -51,6 +51,33 @@ def _image_strided(t):
     return t.contiguous(), c * h * w
 
 
+def _channels_last_view(t):
+    """Element strides (s_n, 1, w * p, p) of an NCHW tensor stored channels-last: the channels of a
+    pixel adjacent, pixels p >= c elements apart, rows dense (a channel slice of a packed
+    ``channels_last`` head output qualifies; p is then the channel count of the whole tensor).
+    None for any other layout and for one that is also planar (n = 1 contiguous, h = w = 1), which
+    ``_image_strided`` handles.  Strides of size-1 dimensions are arbitrary and are not looked at."""
+    n, c, h, w = t.shape
+    st = t.stride()
+    if ((w == 1 or st[3] == 1) and (h == 1 or st[2] == w) and (c == 1 or st[1] == h * w)
+            and (n <= 1 or st[0] >= c * h * w)):
+        return None
+    if w > 1:
+        p = st[3]
+    elif h > 1:
+        p = st[2]
+    else:
+        return None
+    if p < c or (h > 1 and st[2] != w * p) or (c > 1 and st[1] != 1) or (n > 1 and st[0] < h * w * p):
+        return None
+    return (st[0] if n > 1 else h * w * p, 1, w * p, p)
+
+
+def _planar_strides(t, image_stride):
+    _, _, h, w = t.shape
+    return (image_stride, h * w, w, 1)
+
+
 class DecoderEngine(object):
     """One configured decoder bound to one CUDA device."""
 
@@ -338,24 +365,37 @@ class DecoderEngine(object):
         assert hmp.is_cuda == off.is_cuda, 'heat and offset maps must live on the same side'
         self._check_heads(hmp.shape, off.shape, 2, flip)
         args = self._flip_args(flip_tables) if flip else (None, None, None, 0)
-        # Device maps as a reduced-precision network leaves them (bf16 / f16, or channel slices of
-        # one packed head output) are decoded in place on the fused path; anything else becomes
-        # dense float32.
+        # Device maps as a reduced-precision network leaves them (bf16 / f16, channel slices of
+        # one packed head output, channels-last) are decoded in place on the fused path; anything
+        # else becomes dense float32.
         in_place = (not on_host and self._fused and self.thre_hmp > 0 and int(hmp_stride) in (2, 4, 8)
                     and hmp.shape[0] > 0 and hmp.dtype == off.dtype
                     and hmp.dtype in _DTYPES)
         src_hmp, src_off = hmp, off
+        hcl = ocl = None
         if in_place:
-            hmp, hmp_is = _image_strided(hmp)
-            off, off_is = _image_strided(off)
-            in_place = (hmp.dtype != torch.float32 or hmp_is != hmp.shape[1] * hmp.shape[2] * hmp.shape[3]
+            # channels-last maps (a network run in torch.channels_last) are read in place; the
+            # other map of the pair may be planar
+            hcl, ocl = _channels_last_view(hmp), _channels_last_view(off)
+            if hcl is None:
+                hmp, hmp_is = _image_strided(hmp)
+            if ocl is None:
+                off, off_is = _image_strided(off)
+            in_place = (hcl is not None or ocl is not None or hmp.dtype != torch.float32
+                        or hmp_is != hmp.shape[1] * hmp.shape[2] * hmp.shape[3]
                         or off_is != off.shape[1] * off.shape[2] * off.shape[3])
         if not in_place:
             hmp = hmp.contiguous().float()
             off = off.contiguous().float()
         n_in, c, h, w = hmp.shape
         n = n_in // 2 if flip else n_in
-        if in_place:
+        if in_place and (hcl is not None or ocl is not None):
+            fn = self.lib.og_decode_features_dev_strided
+            hs = _lib.int64_array(hcl if hcl is not None else _planar_strides(hmp, hmp_is))
+            os_ = _lib.int64_array(ocl if ocl is not None else _planar_strides(off, off_is))
+            call = (self._h, _ptr(hmp), _ptr(off), _DTYPES[hmp.dtype], hs, os_, n, h, w,
+                    int(hmp_stride), int(off_stride), mode, 1 if flip else 0) + tuple(args)
+        elif in_place:
             fn = self.lib.og_decode_features_dev_ex
             call = (self._h, _ptr(hmp), _ptr(off), _DTYPES[hmp.dtype], hmp_is, off_is, n, h, w,
                     int(hmp_stride), int(off_stride), mode, 1 if flip else 0) + tuple(args)
@@ -501,8 +541,11 @@ class FeaturePlan(object):
         src = (hmp, off)
         if hmp.dtype != off.dtype or hmp.dtype not in _DTYPES:
             hmp, off = hmp.float(), off.float()
-        hmp, hmp_is = _image_strided(hmp)
-        off, off_is = _image_strided(off)
+        hcl, ocl = _channels_last_view(hmp), _channels_last_view(off)
+        if hcl is None:
+            hmp, hmp_is = _image_strided(hmp)
+        if ocl is None:
+            off, off_is = _image_strided(off)
         n_in, _, h, w = hmp.shape
         self.n = n_in // 2 if flip else n_in
         self.eng = eng
@@ -512,9 +555,16 @@ class FeaturePlan(object):
         self.stream_ptr = torch.cuda.current_stream(eng.device).cuda_stream
         plan_id = ctypes.c_int32(-1)
         with torch.cuda.device(eng.device):
-            _lib.check(eng.lib.og_plan_features(
-                eng._h, _ptr(hmp), _ptr(off), _DTYPES[hmp.dtype], hmp_is, off_is, self.n, h, w, int(hmp_stride),
-                int(off_stride), mode, 1 if flip else 0, *args, ctypes.byref(plan_id)))
+            if hcl is not None or ocl is not None:
+                hs = _lib.int64_array(hcl if hcl is not None else _planar_strides(hmp, hmp_is))
+                os_ = _lib.int64_array(ocl if ocl is not None else _planar_strides(off, off_is))
+                _lib.check(eng.lib.og_plan_features_strided(
+                    eng._h, _ptr(hmp), _ptr(off), _DTYPES[hmp.dtype], hs, os_, self.n, h, w, int(hmp_stride),
+                    int(off_stride), mode, 1 if flip else 0, *args, ctypes.byref(plan_id)))
+            else:
+                _lib.check(eng.lib.og_plan_features(
+                    eng._h, _ptr(hmp), _ptr(off), _DTYPES[hmp.dtype], hmp_is, off_is, self.n, h, w,
+                    int(hmp_stride), int(off_stride), mode, 1 if flip else 0, *args, ctypes.byref(plan_id)))
         self._fn = eng.lib.og_plan_launch
         self._handle = eng._h
         self._id = plan_id.value
