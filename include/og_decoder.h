@@ -17,8 +17,8 @@
  *   - every function returns an og_status (0 = OG_OK); og_last_error() gives the
  *     text of the last failure on the calling thread;
  *   - all maps are float32, NCHW, contiguous (og_decode_features_dev_ex also takes
- *     bfloat16 / float16 maps and image-strided views, og_decode_features_dev_strided
- *     channels-last ones as well); "dev" pointers are device
+ *     bfloat16 / float16 maps and image-strided views, og_decode_features_dev_strided and
+ *     og_decode_features_heads_dev_strided channels-last ones as well); "dev" pointers are device
  *     memory of the handle's GPU, "host" pointers are host memory (pinned memory makes
  *     the copies asynchronous and lets the offset maps stay on the host);
  *   - `stream` is the caller's stream: inputs are consumed in its order.  A handle owns one
@@ -256,13 +256,32 @@ int og_decode_features_dev_strided(og_handle *h, const void *hmp_dev, const void
  * their flip-test averages (factory.py:109-113, 141-144) fused in; `cat_flip_offs` scores the limbs
  * on the 4-D vectors [original, mirrored copy] (factory.py:115-127) instead of their average.
  * Either map pointer may be NULL.  Dense float32 maps; same results, bit for bit, as
- * materialising every map and calling og_decode_maps_ex. */
+ * materialising every map and calling og_decode_maps_ex.  Equivalent to
+ * og_decode_features_heads_dev_strided with planar float32 strides. */
 int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float *off_dev,
                                  const float *scale_dev, const float *jitter_dev, int n, int hgt, int w,
                                  int hmp_stride, int off_stride, int resize_mode, int flip_test,
                                  int cat_flip_offs, int use_jitter, const int32_t *kp_flip,
                                  const int32_t *limb_flip, const int32_t *limb_reserve, int n_reserve,
                                  void *stream);
+
+/* og_decode_features_heads_dev on the four maps as a network leaves them: one element type `dtype`
+ * (OG_DTYPE_F32 / BF16 / F16) for all four, each map planar or channels-last with the element
+ * strides and rules of og_decode_features_dev_strided, classified independently (heat: C channels,
+ * offsets: 2L, keypoint scales: C, jitter offsets: 2; n or 2n images with flip_test).  A stride
+ * array may be NULL only when its map is.  Bad strides, types or flags return
+ * OG_ERR_INVALID_ARGUMENT before anything is launched; outside the fused path (strides 2 / 4 / 8,
+ * thre_hmp > 0, fused enabled) the call returns OG_ERR_UNSUPPORTED.  bf16 / f16 values widen exactly
+ * to float32: results are bit-identical to og_decode_features_heads_dev on dense float32 copies. */
+int og_decode_features_heads_dev_strided(og_handle *h, const void *hmp_dev, const void *off_dev,
+                                         const void *scale_dev, const void *jitter_dev, int dtype,
+                                         const int64_t hmp_elem_strides[4], const int64_t off_elem_strides[4],
+                                         const int64_t scale_elem_strides[4],
+                                         const int64_t jitter_elem_strides[4], int n, int hgt, int w,
+                                         int hmp_stride, int off_stride, int resize_mode, int flip_test,
+                                         int cat_flip_offs, int use_jitter, const int32_t *kp_flip,
+                                         const int32_t *limb_flip, const int32_t *limb_reserve,
+                                         int n_reserve, void *stream);
 
 /* A prepared og_decode_features_dev_ex: a network writes its outputs to the same buffers batch
  * after batch, so a caller validates and records the arguments once (og_plan_features, which

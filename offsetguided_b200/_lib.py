@@ -95,6 +95,9 @@ SIGNATURES = {
                             ctypes.POINTER(c_int32_p), ctypes.POINTER(ctypes.c_int32)]),
     'og_decode_features_heads_dev': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i,
                                           _i, _i, c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
+    'og_decode_features_heads_dev_strided': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i64_p, _i64_p, _i64_p, _i64_p,
+                                                  _i, _i, _i, _i, _i, _i, _i, _i, _i,
+                                                  c_int32_p, c_int32_p, c_int32_p, _i, _vp]),
     'og_plan_features': (_i, [_vp, _vp, _vp, _i, ctypes.c_int64, ctypes.c_int64, _i, _i, _i, _i, _i,
                               _i, _i, c_int32_p, c_int32_p, c_int32_p, _i, ctypes.POINTER(ctypes.c_int32)]),
     'og_plan_features_strided': (_i, [_vp, _vp, _vp, _i, _i64_p, _i64_p, _i, _i, _i, _i, _i, _i, _i,

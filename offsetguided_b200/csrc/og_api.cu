@@ -81,11 +81,16 @@ struct GraphKey {
     size_t hmp_plane_stride, hmp_pixel_stride, off_plane_stride, off_pixel_stride;   // planar or channels-last
     int n, hgt, w, stride, mode, flip, coco;
     uint64_t tables_version, buffers_version;
-    const void *scale, *jitter;             // optional heads (og_decode_features_heads_dev)
+    MapView scale, jitter;                  // optional heads (og_decode_features_heads_dev_strided)
     int vector_nd, use_jitter;
+    static bool same_view(const MapView &a, const MapView &b) {
+        return a.ptr == b.ptr && a.dtype == b.dtype && a.image_stride == b.image_stride &&
+               a.plane_stride == b.plane_stride && a.pixel_stride == b.pixel_stride;
+    }
     bool operator==(const GraphKey &o) const {
         return hmp == o.hmp && off == o.off && dtype == o.dtype && coco == o.coco && hmp_image_stride == o.hmp_image_stride &&
-               scale == o.scale && jitter == o.jitter && vector_nd == o.vector_nd && use_jitter == o.use_jitter &&
+               same_view(scale, o.scale) && same_view(jitter, o.jitter) && vector_nd == o.vector_nd &&
+               use_jitter == o.use_jitter &&
                off_image_stride == o.off_image_stride && hmp_plane_stride == o.hmp_plane_stride &&
                hmp_pixel_stride == o.hmp_pixel_stride && off_plane_stride == o.off_plane_stride &&
                off_pixel_stride == o.off_pixel_stride && n == o.n && hgt == o.hgt && w == o.w &&
@@ -659,7 +664,7 @@ int decode_chain(og_handle *h, ResultSlot *slot, const K1Fused &k1, const Offset
                           k1.hmp.plane_stride, k1.hmp.pixel_stride, src.maps.plane_stride, src.maps.pixel_stride,
                           n, k1.h, k1.w, k1.scale, k1.cubic ? 1 : 0, k1.flip ? 1 : 0, slot->emit_coco ? 1 : 0,
                           h->tables_version, slot->buffers_version,
-                          extras ? extras->scale_lr.ptr : nullptr, extras ? extras->jitter_lr.ptr : nullptr,
+                          extras ? extras->scale_lr.maps : MapView(), extras ? extras->jitter_lr.maps : MapView(),
                           extras ? extras->vector_nd : 2, extras ? extras->use_jitter : 0};
     int gi = -1, victim = 0;
     for (int i = 0; i < kGraphsPerSlot; ++i) {
@@ -1206,42 +1211,6 @@ int og_decode_features_dev(og_handle *h, const float *hmp_dev, const float *off_
                                 resize_mode, flip_test, s, true);
 }
 
-int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float *off_dev,
-                                 const float *scale_dev, const float *jitter_dev, int n, int hgt, int w,
-                                 int hmp_stride, int off_stride, int resize_mode, int flip_test,
-                                 int cat_flip_offs, int use_jitter, const int32_t *kp_flip,
-                                 const int32_t *limb_flip, const int32_t *limb_reserve, int n_reserve,
-                                 void *stream) {
-    OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_heads_dev: null pointer");
-    OG_REQUIRE(!cat_flip_offs || flip_test, "cat_flip_offs concatenates the mirrored copy's offsets: it needs flip_test");
-    OG_REQUIRE(!(cat_flip_offs && jitter_dev && use_jitter),
-               "jitter refinement of 4-D offset vectors is undefined (it raises in the reference too)");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
-                              limb_flip, limb_reserve, n_reserve));
-    const og_config &c = h->cfg;
-    if (!(h->fused_enabled && c.thre_hmp > 0.0f && fused_supported(n, c.n_keypoints, hmp_stride, hgt, w))) {
-        set_error("og_decode_features_heads_dev needs the fused path (stride 2, 4 or 8, thre_hmp > 0, fused "
-                  "enabled); resize the maps and call og_decode_maps_ex");
-        return OG_ERR_UNSUPPORTED;
-    }
-    ResultSlot *slot = nullptr;
-    OG_TRY(acquire_slot(h, nullptr, &slot));
-    const size_t hw = (size_t)hgt * w;
-    const int H = hgt * hmp_stride, W = w * hmp_stride;
-    OG_TRY(check_maps(n, H, W, c.n_keypoints));
-    K1Fused k1 = {dense_f32(hmp_dev, (size_t)c.n_keypoints * hw, hw), hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
-    OffsetSource src = {dense_f32(off_dev, (size_t)2 * c.n_limbs * hw, hw), hgt, w, off_stride, flip_test ? 1 : 0, n};
-    LimbExtras ex = {};
-    ex.vector_nd = cat_flip_offs ? 4 : 2;
-    ex.use_jitter = use_jitter ? 1 : 0;
-    // keypoint scales are resized like the heat maps (x off_stride, inter_mode), jitter offsets
-    // bilinearly x hmp_stride (factory.py:80-88)
-    ex.scale_lr = HeadSource{scale_dev, hgt, w, off_stride, resize_mode == 1 ? 1 : 0};
-    ex.jitter_lr = HeadSource{jitter_dev, hgt, w, hmp_stride, 0};
-    return decode_chain(h, slot, k1, src, n, H, W, s, &ex);
-}
-
 namespace {
 
 // The view of one map from its element strides in (image, channel, row, column) order: planar
@@ -1271,22 +1240,29 @@ int map_view(const char *name, const void *ptr, int dtype, const int64_t st[4], 
     return OG_OK;
 }
 
-// og_decode_features_dev_strided behind its argument checks (also the body of a plan launch)
+// og_decode_features_dev_strided / og_decode_features_heads_dev_strided behind their argument checks
+// (also the body of a plan launch); `extras`: the optional heads and flags, which only the fused
+// path decodes
 int decode_dev_views(og_handle *h, const MapView &hv, const MapView &ov, int n, int hgt, int w, int hmp_stride,
-                     int off_stride, int resize_mode, int flip_test, cudaStream_t s) {
+                     int off_stride, int resize_mode, int flip_test, cudaStream_t s,
+                     const LimbExtras *extras = nullptr) {
     const og_config &c = h->cfg;
     const size_t hw = (size_t)hgt * w;
     const size_t hmp_img = (size_t)c.n_keypoints * hw, off_img = (size_t)2 * c.n_limbs * hw;
-    if (hv.dtype == OG_DTYPE_F32 && !hv.is_channels_last() && !ov.is_channels_last() && hv.image_stride == hmp_img &&
-        ov.image_stride == off_img) {
+    if (!extras && hv.dtype == OG_DTYPE_F32 && !hv.is_channels_last() && !ov.is_channels_last() &&
+        hv.image_stride == hmp_img && ov.image_stride == off_img) {
         ResultSlot *slot = nullptr;
         OG_TRY(acquire_slot(h, nullptr, &slot));
         return decode_features_impl(h, slot, static_cast<const float *>(hv.ptr), static_cast<const float *>(ov.ptr),
                                     n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, s, true);
     }
     if (!(h->fused_enabled && c.thre_hmp > 0.0f && fused_supported(n, c.n_keypoints, hmp_stride, hgt, w))) {
-        set_error("og_decode_features_dev_ex: bf16 / strided maps need the fused path (stride 2, 4 or 8, "
-                  "thre_hmp > 0, fused enabled); convert to dense float32 and call og_decode_features_dev");
+        if (extras)
+            set_error("og_decode_features_heads_dev needs the fused path (stride 2, 4 or 8, thre_hmp > 0, fused "
+                      "enabled); resize the maps and call og_decode_maps_ex");
+        else
+            set_error("og_decode_features_dev_ex: bf16 / strided maps need the fused path (stride 2, 4 or 8, "
+                      "thre_hmp > 0, fused enabled); convert to dense float32 and call og_decode_features_dev");
         return OG_ERR_UNSUPPORTED;
     }
     ResultSlot *slot = nullptr;
@@ -1295,7 +1271,7 @@ int decode_dev_views(og_handle *h, const MapView &hv, const MapView &ov, int n, 
     OG_TRY(check_maps(n, H, W, c.n_keypoints));
     K1Fused k1 = {hv, hgt, w, hmp_stride, resize_mode == 1, flip_test != 0};
     OffsetSource src = {ov, hgt, w, off_stride, flip_test ? 1 : 0, n};
-    return decode_chain(h, slot, k1, src, n, H, W, s);
+    return decode_chain(h, slot, k1, src, n, H, W, s, extras);
 }
 
 int check_dtype(int dtype) {
@@ -1359,6 +1335,59 @@ int og_decode_features_dev_ex(og_handle *h, const void *hmp_dev, const void *off
     return og_decode_features_dev_strided(h, hmp_dev, off_dev, dtype, hs, os, n, hgt, w, hmp_stride, off_stride,
                                           resize_mode, flip_test, kp_flip, limb_flip, limb_reserve, n_reserve,
                                           stream);
+}
+
+int og_decode_features_heads_dev_strided(og_handle *h, const void *hmp_dev, const void *off_dev, const void *scale_dev,
+                                         const void *jitter_dev, int dtype, const int64_t hmp_elem_strides[4],
+                                         const int64_t off_elem_strides[4], const int64_t scale_elem_strides[4],
+                                         const int64_t jitter_elem_strides[4], int n, int hgt, int w, int hmp_stride,
+                                         int off_stride, int resize_mode, int flip_test, int cat_flip_offs,
+                                         int use_jitter, const int32_t *kp_flip, const int32_t *limb_flip,
+                                         const int32_t *limb_reserve, int n_reserve, void *stream) {
+    OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_heads_dev: null pointer");
+    OG_REQUIRE(!cat_flip_offs || flip_test, "cat_flip_offs concatenates the mirrored copy's offsets: it needs flip_test");
+    OG_REQUIRE(!(cat_flip_offs && jitter_dev && use_jitter),
+               "jitter refinement of 4-D offset vectors is undefined (it raises in the reference too)");
+    OG_TRY(check_dtype(dtype));
+    OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
+                              limb_flip, limb_reserve, n_reserve));
+    MapView hv, ov, sv, jv;
+    OG_TRY(feature_views(h, hmp_dev, off_dev, dtype, hmp_elem_strides, off_elem_strides, n, hgt, w, flip_test, &hv,
+                         &ov));
+    const int images = flip_test ? 2 * n : n;
+    if (scale_dev)
+        OG_TRY(map_view("scale_elem_strides", scale_dev, dtype, scale_elem_strides, h->cfg.n_keypoints, images, hgt,
+                        w, &sv));
+    if (jitter_dev)
+        OG_TRY(map_view("jitter_elem_strides", jitter_dev, dtype, jitter_elem_strides, 2, images, hgt, w, &jv));
+    LimbExtras ex = {};
+    ex.vector_nd = cat_flip_offs ? 4 : 2;
+    ex.use_jitter = use_jitter ? 1 : 0;
+    // keypoint scales are resized like the heat maps (x off_stride, inter_mode), jitter offsets
+    // bilinearly x hmp_stride (factory.py:80-88)
+    ex.scale_lr = HeadSource{sv, hgt, w, off_stride, resize_mode == 1 ? 1 : 0};
+    ex.jitter_lr = HeadSource{jv, hgt, w, hmp_stride, 0};
+    return decode_dev_views(h, hv, ov, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test,
+                            static_cast<cudaStream_t>(stream), &ex);
+}
+
+int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float *off_dev,
+                                 const float *scale_dev, const float *jitter_dev, int n, int hgt, int w,
+                                 int hmp_stride, int off_stride, int resize_mode, int flip_test,
+                                 int cat_flip_offs, int use_jitter, const int32_t *kp_flip,
+                                 const int32_t *limb_flip, const int32_t *limb_reserve, int n_reserve,
+                                 void *stream) {
+    OG_REQUIRE(h, "og_decode_features_heads_dev: null pointer");
+    OG_TRY(check_maps(n, hgt, w, h->cfg.n_keypoints));
+    int64_t hs[4], os[4], ss[4], js[4];
+    OG_TRY(planar_strides("hmp", 0, h->cfg.n_keypoints, hgt, w, hs));
+    OG_TRY(planar_strides("off", 0, 2 * h->cfg.n_limbs, hgt, w, os));
+    OG_TRY(planar_strides("scale", 0, h->cfg.n_keypoints, hgt, w, ss));
+    OG_TRY(planar_strides("jitter", 0, 2, hgt, w, js));
+    return og_decode_features_heads_dev_strided(h, hmp_dev, off_dev, scale_dev, jitter_dev, OG_DTYPE_F32, hs, os,
+                                                scale_dev ? ss : nullptr, jitter_dev ? js : nullptr, n, hgt, w,
+                                                hmp_stride, off_stride, resize_mode, flip_test, cat_flip_offs,
+                                                use_jitter, kp_flip, limb_flip, limb_reserve, n_reserve, stream);
 }
 
 int og_plan_features_strided(og_handle *h, const void *hmp_dev, const void *off_dev, int dtype,

@@ -171,11 +171,12 @@ struct OffsetSource {
     int flip, n;                    // flip: maps = n originals then n mirrored copies
 };
 
-// An optional head at NETWORK resolution (float32, dense [n or 2n][channels][h][w]; the flip layout
-// and image count are those of the OffsetSource of the call): K2 interpolates it at the few
-// pixels it needs instead of reading a materialised x scale map.
+// An optional head at NETWORK resolution ([n or 2n][channels][h][w], planar or channels-last, the
+// element type of the call's other maps; the flip layout and image count are those of the
+// OffsetSource of the call): K2 interpolates it at the few pixels it needs instead of reading a
+// materialised x scale map.
 struct HeadSource {
-    const float *ptr;       // nullptr: head not present
+    MapView maps;           // maps.ptr == nullptr: head not present
     int h, w, scale;
     int cubic;              // interpolation of the reference's resize (factory.py:80-88)
 };

@@ -95,16 +95,26 @@ __device__ __forceinline__ float sample_offset(const OffsetSource &src, const Fl
     return sample_offset_t<float>(src, ft, img, l, comp, cat, X, Y);
 }
 
-// Channel ch of an optional head (keypoint scales: channels = C, mirrored partner ft.kp[ch],
-// factory.py:141-144; jitter offsets: channels = 2, partner = the same channel with x negated,
+// Channel ch of an optional head (keypoint scales: mirrored partner = channel ft.kp[ch] of image
+// n + img, factory.py:141-144; jitter offsets: partner = the same channel with x negated,
 // factory.py:109-113) at full-resolution pixel (X, Y).
-__device__ __forceinline__ float sample_head(const HeadSource &hs, const OffsetSource &src, int img, int channels,
-                                             int ch, int partner, bool negate_partner, int X, int Y) {
-    const size_t hw = (size_t)hs.h * hs.w;
-    const float *a = hs.ptr + ((size_t)img * channels + ch) * hw;
-    const float *b = src.flip ? hs.ptr + ((size_t)(src.n + img) * channels + partner) * hw : nullptr;
-    return sample_lowres(a, b, src.flip ? kFlipAverage : kFlipNone, negate_partner, hs.h, hs.w, (size_t)1, hs.scale,
-                         hs.cubic != 0, X, Y);
+template <typename T>
+__device__ __forceinline__ float sample_head_t(const HeadSource &hs, const OffsetSource &src, int img, int ch,
+                                               int partner, bool negate_partner, int X, int Y) {
+    const T *base = static_cast<const T *>(hs.maps.ptr);
+    const T *a = base + (size_t)img * hs.maps.image_stride + (size_t)ch * hs.maps.plane_stride;
+    const T *b = src.flip ? base + (size_t)(src.n + img) * hs.maps.image_stride +
+                                (size_t)partner * hs.maps.plane_stride
+                          : nullptr;
+    return sample_lowres(a, b, src.flip ? kFlipAverage : kFlipNone, negate_partner, hs.h, hs.w,
+                         hs.maps.pixel_stride, hs.scale, hs.cubic != 0, X, Y);
+}
+
+__device__ __forceinline__ float sample_head(const HeadSource &hs, const OffsetSource &src, int img, int ch,
+                                             int partner, bool negate_partner, int X, int Y) {
+    if (hs.maps.dtype == OG_DTYPE_BF16) return sample_head_t<__nv_bfloat16>(hs, src, img, ch, partner, negate_partner, X, Y);
+    if (hs.maps.dtype == OG_DTYPE_F16) return sample_head_t<__half>(hs, src, img, ch, partner, negate_partner, X, Y);
+    return sample_head_t<float>(hs, src, img, ch, partner, negate_partner, X, Y);
 }
 
 // Tensor.norm over 4 components as ATen's CPU kernel evaluates it (probed) is a plain left-to-right
@@ -167,8 +177,8 @@ limb_score_kernel(const float *__restrict__ det_score, const int32_t *__restrict
         if (t.index >= 0) {
             if (scales != nullptr)
                 t.scale = __ldg(scales + ((size_t)n * C + jt) * HW + t.index);   // collect.py:114
-            else if (ex.scale_lr.ptr != nullptr)
-                t.scale = sample_head(ex.scale_lr, src, n, C, jt, ft.kp[jt], false, t.index % W, t.index / W);
+            else if (ex.scale_lr.maps.ptr != nullptr)
+                t.scale = sample_head(ex.scale_lr, src, n, jt, ft.kp[jt], false, t.index % W, t.index / W);
         }
         s_to[k] = t;
     }
@@ -196,8 +206,8 @@ limb_score_kernel(const float *__restrict__ det_score, const int32_t *__restrict
         }
         if (scales != nullptr)
             scale1 = __ldg(scales + ((size_t)n * C + jf) * HW + idx1);
-        else if (ex.scale_lr.ptr != nullptr)
-            scale1 = sample_head(ex.scale_lr, src, n, C, jf, ft.kp[jf], false, idx1 % W, idx1 / W);
+        else if (ex.scale_lr.maps.ptr != nullptr)
+            scale1 = sample_head(ex.scale_lr, src, n, jf, ft.kp[jf], false, idx1 % W, idx1 / W);
     }
     __syncthreads();
 
@@ -207,10 +217,10 @@ limb_score_kernel(const float *__restrict__ det_score, const int32_t *__restrict
         const float gx2 = __fadd_rn(x1, __fmul_rn(ox2, resize_factor));
         const float gy2 = __fadd_rn(y1, __fmul_rn(oy2, resize_factor));
         // jitter-offset component `comp` at decode-resolution pixel (row py, column px)
-        const bool have_jitter = ex.jomps != nullptr || ex.jitter_lr.ptr != nullptr;
+        const bool have_jitter = ex.jomps != nullptr || ex.jitter_lr.maps.ptr != nullptr;
         auto jitter_at = [&](int comp, int px, int py) {
             if (ex.jomps != nullptr) return __ldg(ex.jomps + ((size_t)n * 2 + comp) * HW + (size_t)py * W + px);
-            return sample_head(ex.jitter_lr, src, n, 2, comp, comp, comp == 0, px, py);
+            return sample_head(ex.jitter_lr, src, n, comp, comp, comp == 0, px, py);
         };
         if (have_jitter && ex.use_jitter && !kFour) {
             // jitter refinement of the guided point (collect.py:158-165), including the

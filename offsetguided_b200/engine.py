@@ -40,14 +40,24 @@ def _view(pointer, ctype, count, dtype):
     return np.frombuffer((ctype * count).from_address(ctypes.addressof(pointer.contents)), dtype=dtype)
 
 
+def _planar_image_stride(t):
+    """Elements between images of an NCHW tensor whose planes are dense and contiguous within an
+    image (a channel slice of a packed head output qualifies), else None."""
+    n, c, h, w = t.shape
+    st = t.stride()
+    if st[3] == 1 and st[2] == w and st[1] == h * w and (n <= 1 or st[0] >= c * h * w):
+        return st[0] if n > 1 else c * h * w
+    return None
+
+
 def _image_strided(t):
     """(tensor, elements between images) for an NCHW tensor whose planes are dense and contiguous
     within an image (a channel slice of a packed head output qualifies); other layouts are
     made contiguous first."""
+    image_stride = _planar_image_stride(t)
+    if image_stride is not None:
+        return t, image_stride
     n, c, h, w = t.shape
-    st = t.stride()
-    if st[3] == 1 and st[2] == w and st[1] == h * w and (n <= 1 or st[0] >= c * h * w):
-        return t, (st[0] if n > 1 else c * h * w)
     return t.contiguous(), c * h * w
 
 
@@ -76,6 +86,37 @@ def _channels_last_view(t):
 def _planar_strides(t, image_stride):
     _, _, h, w = t.shape
     return (image_stride, h * w, w, 1)
+
+
+def _heads_in_place(maps):
+    """How decode_features_heads hands over ``maps`` = (heat, offsets, keypoint scales or None,
+    jitter offsets or None): the element strides of each map (None for an absent head) when the
+    library can read all of them where they are, or None when they are converted to dense float32
+    first.  In place: CUDA tensors of one supported element type, each planar with dense planes
+    (image-strided, ``_planar_image_stride``) or channels-last (``_channels_last_view``), not all of
+    them dense float32 already."""
+    present = [t for t in maps if t is not None]
+    if not all(getattr(t, 'is_cuda', False) for t in present) or present[0].shape[0] == 0:
+        return None
+    dtype = present[0].dtype
+    if dtype not in _DTYPES or any(t.dtype != dtype for t in present):
+        return None
+    strides, dense = [], dtype == torch.float32
+    for t in maps:
+        if t is None:
+            strides.append(None)
+            continue
+        cl = _channels_last_view(t)
+        if cl is not None:
+            strides.append(cl)
+            dense = False
+            continue
+        image_stride = _planar_image_stride(t)
+        if image_stride is None:
+            return None
+        strides.append(_planar_strides(t, image_stride))
+        dense = dense and image_stride == t.shape[1] * t.shape[2] * t.shape[3]
+    return None if dense else strides
 
 
 class DecoderEngine(object):
@@ -418,30 +459,34 @@ class DecoderEngine(object):
         """decode_features with the optional heads on the fused path: keypoint-scale maps and
         jitter-offset maps at NETWORK resolution are interpolated by K2 at the candidate pixels
         (flip-test averages fused in), ``cat_flip_offs`` scores limbs on the 4-D [original,
-        mirrored] offset vectors.  Device-resident maps (anything else is converted to dense
-        float32 on the device first)."""
+        mirrored] offset vectors.  Device-resident maps of one element type (f32 / bf16 / f16),
+        each planar with dense planes or channels-last, are read in place (``_heads_in_place``);
+        anything else is converted to dense float32 on the device first."""
         flip = flip_tables is not None
         self._check_heads(hmp.shape, off.shape, 2, flip)
         mode = {'bilinear': 0, 'bicubic': 1}[resize_mode]
-        hmp = as_cuda_f32(hmp, self.device)
-        off = as_cuda_f32(off, self.device)
         n_in, c, h, w = hmp.shape
-        keep = [hmp, off]
         for t, ch in ((scales, c), (jomps, 2)):
             if t is not None and tuple(t.shape) != (n_in, ch, h, w):
                 raise ValueError('optional head of shape %s, expected %s' % (tuple(t.shape), (n_in, ch, h, w)))
-        scales = as_cuda_f32(scales, self.device) if scales is not None else None
-        jomps = as_cuda_f32(jomps, self.device) if jomps is not None else None
-        keep += [scales, jomps]
         args = self._flip_args(flip_tables) if flip else (None, None, None, 0)
         n = n_in // 2 if flip else n_in
+        maps = (hmp, off, scales, jomps)
+        strides = _heads_in_place(maps)
+        if strides is None:
+            maps = tuple(as_cuda_f32(t, self.device) if t is not None else None for t in maps)
+        ptrs = tuple(_ptr(t) if t is not None else None for t in maps)
+        flags = (n, h, w, int(hmp_stride), int(off_stride), mode, 1 if flip else 0, 1 if cat_flip_offs else 0,
+                 1 if use_jitter else 0) + tuple(args)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.og_decode_features_heads_dev(
-                self._h, _ptr(hmp), _ptr(off), _ptr(scales) if scales is not None else None,
-                _ptr(jomps) if jomps is not None else None, n, h, w, int(hmp_stride), int(off_stride), mode,
-                1 if flip else 0, 1 if cat_flip_offs else 0, 1 if use_jitter else 0, *args,
-                _stream_ptr(self.device)))
-        return self._finish(tuple(keep), fetch, n)
+            if strides is None:
+                st = self.lib.og_decode_features_heads_dev(self._h, *ptrs, *flags, _stream_ptr(self.device))
+            else:
+                st_arrays = tuple(_lib.int64_array(s) if s is not None else None for s in strides)
+                st = self.lib.og_decode_features_heads_dev_strided(self._h, *ptrs, _DTYPES[hmp.dtype], *st_arrays,
+                                                                   *flags, _stream_ptr(self.device))
+            _lib.check(st)
+        return self._finish(maps, fetch, n)
 
     def plan_features(self, hmp, off, hmp_stride, off_stride, resize_mode='bicubic', flip_tables=None):
         """A prepared decode of DEVICE-resident network-resolution maps for callers that decode the
