@@ -215,31 +215,41 @@ def oracle_dets(heat_lo, scale, mode, k):
 
 
 # --------------------------------------------------------------------------- scan model
-def scan_flags(a, b, scale, mode, variant='exact'):
+def scan_flags(a, b, scale, mode, variant='exact', thre=THRE, factor=None):
     """numpy model of amax_scan_kernel's vector path for one plane: the work blocks it flags.
-    `a` is the plane, `b` the mirrored partner plane of a flip-test (None without flip).
+    `a` is the plane, `b` the mirrored partner plane of a flip-test (None without flip).  The
+    block flags of the scalar path and of amax_scan_nhwc_kernel are the same; a width that is not
+    a multiple of 4 cells is modelled without lane order.
     `variant` models a kernel defect:
       'no_abs'   the scan tests v instead of |v|;
       'limit'    the scan's limit is thre instead of thre / 1.95 (bicubic) or thre / 1.001;
+      'halo'     both halos one cell short (1 for bicubic, 0 for bilinear);
       'lanes01'  lanes 0 and 1 of each 4-cell load swapped (both inputs);
       'halves'   the two 2-cell halves of each 4-cell load swapped (both inputs);
-      'mirror'   the mirrored copy's lanes 0 and 3 paired with the wrong cells."""
+      'mirror'   the mirrored copy's lanes 0 and 3 paired with the wrong cells.
+    `factor` replaces the bound factor of the limit thre / factor (1.95 bicubic, 1.001 bilinear)."""
     h, w = a.shape
     cubic = mode == 'bicubic'
-    halo = 2 if cubic else 1
-    limit = np.float32(THRE) if variant == 'limit' else np.float32(THRE / (1.95 if cubic else 1.001))
+    halo = (2 if cubic else 1) - (variant == 'halo')
+    if factor is None:
+        factor = 1.95 if cubic else 1.001
+    # og_fused.cu scan_limit: a float32 division
+    limit = np.float32(thre) if variant == 'limit' else np.float32(thre) / np.float32(factor)
     perm = {'lanes01': (1, 0, 2, 3), 'halves': (2, 3, 0, 1)}.get(variant, (0, 1, 2, 3))
-    g = a.reshape(h, w // KSUB, KSUB)
-    va = g[:, :, list(perm)]
-    if b is None:
-        f = va
+    if w % KSUB:
+        assert perm == (0, 1, 2, 3) and variant != 'mirror', variant
+        f = a if b is None else ((a + b[:, ::-1]) * np.float32(0.5)).astype(np.float32)
     else:
-        # vb[i] = b[w - 4 - x0 + perm[i]]: the mirrored group, in load order
-        gb = b[:, ::-1].reshape(h, w // KSUB, KSUB)[:, :, ::-1]        # gb[.., x0 / 4, i] = b[w - 4 - x0 + i]
-        vb = gb[:, :, list(perm)]
-        pair = (0, 2, 1, 3) if variant == 'mirror' else (3, 2, 1, 0)
-        f = ((va + vb[:, :, list(pair)]) * np.float32(0.5)).astype(np.float32)
-    f = f.reshape(h, w)
+        va = a.reshape(h, w // KSUB, KSUB)[:, :, list(perm)]
+        if b is None:
+            f = va
+        else:
+            # vb[i] = b[w - 4 - x0 + perm[i]]: the mirrored group, in load order
+            gb = b[:, ::-1].reshape(h, w // KSUB, KSUB)[:, :, ::-1]        # gb[.., x0 / 4, i] = b[w - 4 - x0 + i]
+            vb = gb[:, :, list(perm)]
+            pair = (0, 2, 1, 3) if variant == 'mirror' else (3, 2, 1, 0)
+            f = ((va + vb[:, :, list(pair)]) * np.float32(0.5)).astype(np.float32)
+        f = f.reshape(h, w)
     hot = (f >= limit) if variant == 'no_abs' else ~(np.abs(f) < limit)
     bw = 32 // scale
     bxs, bys = (w + bw - 1) // bw, (h + BLOCK_H - 1) // BLOCK_H
