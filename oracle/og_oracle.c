@@ -296,11 +296,18 @@ int oc_group_image(const float *limbs, int c, int l, int k, const int32_t *from,
             if (use_scale) lim = (r[12] != r[12]) ? r[12] : (dist_max > r[12] ? dist_max : r[12]);
             if (r[8] < lim && r[0] > 0 && r[4] > 0 && r[3] > 0 && r[1] > 0) rows[nv++] = q;
         }
-        for (int i = 1; i < nv; ++i) {                   /* stable sort, limb score desc (:232) */
+        /* stable sort, limb score desc (:232); NaN scores (0 / 0 at min_len = 0) after every
+         * number, in row order: the stable form of np.argsort(-s) */
+        for (int i = 1; i < nv; ++i) {
             const int q = rows[i];
             const float s = conns[q * LIMB_COLS + 10];
             int j = i - 1;
-            while (j >= 0 && conns[rows[j] * LIMB_COLS + 10] < s) { rows[j + 1] = rows[j]; --j; }
+            while (j >= 0 && s == s) {
+                const float t = conns[rows[j] * LIMB_COLS + 10];
+                if (!(t != t || t < s)) break;
+                rows[j + 1] = rows[j];
+                --j;
+            }
             rows[j + 1] = q;
         }
         int kk = 0;

@@ -146,10 +146,15 @@ def _norm4(a, b, c, d):
 
 def generate_limbs(hmps_hr, offs_hr, skeleton, topk, thre_hmp, min_len,
                    hmp_s=4, off_s=4, scmps_hr=None, return_dets=False, jomps_hr=None,
-                   use_jitter=True, vector_nd=2):
+                   use_jitter=True, vector_nd=2, unrefined_off_plane=False):
     """decoder/collect.py:62-236 with include_scale / include_jitter_offset off
     unless ``scmps_hr`` (the scale gather of :111-116, 257-262) / ``jomps_hr`` (jitter offsets,
     :127-138, 158-165, 213-218) are given; ``vector_nd = 4`` is the cat_flip_offs layout.
+
+    The jitter refinement indexes the (H, W) jitter plane as [x, y] = [row, col] after a bounds
+    check against (W, H), so on maps with H != W the reference raises IndexError for a guided
+    point with x >= H or y >= W; so does this oracle, unless ``unrefined_off_plane`` is set: such
+    points are then left unrefined, as the CUDA decoder leaves them.
 
     Returns limbs (N, L, K, 13) float32 =
     [x1, y1, v1, x2, y2, v2, ind1, ind2, min_dist, len, limb_score, scale1, scale2].
@@ -190,6 +195,8 @@ def generate_limbs(hmps_hr, offs_hr, skeleton, topk, thre_hmp, min_len,
                     for k in range(topk):
                         gx_, gy_ = int(gi[i, j, k, 0]), int(gi[i, j, k, 1])
                         if 0 <= gx_ < w and 0 <= gy_ < h:
+                            if unrefined_off_plane and not (gx_ < h and gy_ < w):
+                                continue
                             guid[i, j, k] += jm[i, :, gx_, gy_]               # [x, y] as [row, col]
     else:
         jit_f = jit_t = None
@@ -249,8 +256,12 @@ def valid_limb_rows(conns, dist_max, use_scale):
 
 def delete_reconns(conns, rows):
     """decoder/group.py:222-240 — sort by limb score desc (canonical: stable) and
-    keep the best row per distinct to-joint id."""
-    rows = sorted(rows, key=lambda k: -float(conns[k, 10]))   # Python sort is stable
+    keep the best row per distinct to-joint id.  A NaN score (0 / 0 at min_len = 0) ranks after
+    every number, NaN rows in row order: the stable form of the reference's np.argsort(-s)."""
+    def key(k):
+        s = float(conns[k, 10])
+        return (1, 0.0) if s != s else (0, -s)
+    rows = sorted(rows, key=key)                              # Python sort is stable
     seen, kept = set(), []
     for k in rows:
         t = int(conns[k, 7])
@@ -531,10 +542,11 @@ def generate_poses(hmps, offs, skeleton, n_keypoints, *, topk, thre_hmp, min_len
                    sort_dim=2, dist_max=20, use_scale=True, hmp_stride=4, off_stride=4,
                    resize_mode='bicubic', flip_test=False, kp_flips=None, limb_flips=None,
                    limb_reserve=None, return_limbs=False, scmps=None, jomps=None, use_jitter=True,
-                   cat_flip_offs=False):
+                   cat_flip_offs=False, unrefined_off_plane=False):
     """decoder/factory.py:52-96 on network-resolution maps: optional flip fusion, x stride
     resize, limb collection, greedy grouping; ``scmps`` / ``jomps`` are the optional
-    keypoint-scale and jitter-offset heads, ``cat_flip_offs`` the 4-D offset variant."""
+    keypoint-scale and jitter-offset heads, ``cat_flip_offs`` the 4-D offset variant;
+    ``unrefined_off_plane``: see generate_limbs."""
     vector_nd = 2
     if flip_test:
         if cat_flip_offs:
@@ -553,7 +565,8 @@ def generate_poses(hmps, offs, skeleton, n_keypoints, *, topk, thre_hmp, min_len
     jomps_hr = resize(jomps, hmp_stride, 'bilinear') if jomps is not None else None
     limbs = generate_limbs(hmps_hr, offs_hr, skeleton, topk, thre_hmp, min_len,
                            hmp_stride, off_stride, scmps_hr=scmps_hr, jomps_hr=jomps_hr,
-                           use_jitter=use_jitter, vector_nd=vector_nd)
+                           use_jitter=use_jitter, vector_nd=vector_nd,
+                           unrefined_off_plane=unrefined_off_plane)
     poses = [group_skeletons(l, skeleton, n_keypoints, person_thre, sort_dim, dist_max, use_scale)
              for l in limbs]
     if return_limbs:
