@@ -336,7 +336,9 @@ int og_fetch_result(og_handle *h, og_result *out);
  * (meta['offset'], meta['scale']).  The grouping kernel then also writes, for every person,
  * x' = around((x + offset_x) / scale_x, 2), y' likewise, flag = (x' > 0 or y' > 0) per keypoint
  * and score = sum(v) / C, with the reference's rounding (float64 steps rounded to float32, numpy's
- * float32 around, float64 score); og_fetch_result exposes them next to the poses. */
+ * float32 around, float64 score); og_fetch_result exposes them next to the poses.  The frames
+ * belong to that next call whether it runs or is refused: a refused call drops them, so the call
+ * after it has no frames unless they are staged again. */
 int og_set_frames(og_handle *h, const double *frames_host, int n);
 int og_fetch_poses(og_handle *h, const float **poses_host, const int32_t **offset_host,
                    const int32_t **count_host, int32_t *total_rows);

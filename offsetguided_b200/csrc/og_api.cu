@@ -800,6 +800,16 @@ int decode_features_impl(og_handle *h, ResultSlot *slot, const float *hmp, const
     return decode_core(h, slot, cur_h, nullptr, cur_o, nullptr, nullptr, n, H, W, s);
 }
 
+// The frames staged by og_set_frames belong to the next decode call, whether that call runs or is
+// refused: one on every og_decode_* entry point drops them on return, so that a refused call does
+// not hand its frames to the call after it (begin_call has taken them over when the call runs).
+struct StagedFramesOfCall {
+    og_handle *h;
+    ~StagedFramesOfCall() {
+        if (h) h->staged_n = -1;
+    }
+};
+
 int check_feature_args(og_handle *h, int n, int hgt, int w, int hmp_stride, int off_stride,
                        int resize_mode, int flip_test, const int32_t *kp_flip,
                        const int32_t *limb_flip, const int32_t *limb_reserve, int n_reserve) {
@@ -1174,6 +1184,7 @@ int og_resize_f32(const float *in_dev, float *out_dev, int planes, int hgt, int 
 
 int og_decode_maps(og_handle *h, const float *heat_dev, const float *offs_dev,
                    const float *scales_dev, int n, int hgt, int w, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (heat_dev && offs_dev)), "og_decode_maps: null pointer");
     OG_TRY(check_device(h));
     ResultSlot *slot = nullptr;
@@ -1185,6 +1196,7 @@ int og_decode_maps(og_handle *h, const float *heat_dev, const float *offs_dev,
 int og_decode_maps_ex(og_handle *h, const float *heat_dev, const float *offs_dev,
                       const float *scales_dev, const float *jomps_dev, int vector_nd, int use_jitter,
                       int n, int hgt, int w, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (heat_dev && offs_dev)), "og_decode_maps_ex: null pointer");
     OG_REQUIRE(vector_nd == 2 || vector_nd == 4, "vector_nd must be 2 or 4");
     OG_REQUIRE(!(vector_nd == 4 && jomps_dev && use_jitter),
@@ -1201,6 +1213,7 @@ int og_decode_features_dev(og_handle *h, const float *hmp_dev, const float *off_
                            int w, int hmp_stride, int off_stride, int resize_mode, int flip_test,
                            const int32_t *kp_flip, const int32_t *limb_flip,
                            const int32_t *limb_reserve, int n_reserve, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_dev: null pointer");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
@@ -1309,6 +1322,7 @@ int og_decode_features_dev_strided(og_handle *h, const void *hmp_dev, const void
                                    int hgt, int w, int hmp_stride, int off_stride, int resize_mode, int flip_test,
                                    const int32_t *kp_flip, const int32_t *limb_flip,
                                    const int32_t *limb_reserve, int n_reserve, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_dev_strided: null pointer");
     OG_TRY(check_dtype(dtype));
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
@@ -1325,6 +1339,7 @@ int og_decode_features_dev_ex(og_handle *h, const void *hmp_dev, const void *off
                               int w, int hmp_stride, int off_stride, int resize_mode, int flip_test,
                               const int32_t *kp_flip, const int32_t *limb_flip,
                               const int32_t *limb_reserve, int n_reserve, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_dev_ex: null pointer");
     OG_TRY(check_dtype(dtype));
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,
@@ -1344,6 +1359,7 @@ int og_decode_features_heads_dev_strided(og_handle *h, const void *hmp_dev, cons
                                          int off_stride, int resize_mode, int flip_test, int cat_flip_offs,
                                          int use_jitter, const int32_t *kp_flip, const int32_t *limb_flip,
                                          const int32_t *limb_reserve, int n_reserve, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (hmp_dev && off_dev)), "og_decode_features_heads_dev: null pointer");
     OG_REQUIRE(!cat_flip_offs || flip_test, "cat_flip_offs concatenates the mirrored copy's offsets: it needs flip_test");
     OG_REQUIRE(!(cat_flip_offs && jitter_dev && use_jitter),
@@ -1377,6 +1393,7 @@ int og_decode_features_heads_dev(og_handle *h, const float *hmp_dev, const float
                                  int cat_flip_offs, int use_jitter, const int32_t *kp_flip,
                                  const int32_t *limb_flip, const int32_t *limb_reserve, int n_reserve,
                                  void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h, "og_decode_features_heads_dev: null pointer");
     OG_TRY(check_maps(n, hgt, w, h->cfg.n_keypoints));
     int64_t hs[4], os[4], ss[4], js[4];
@@ -1436,6 +1453,7 @@ int og_plan_features(og_handle *h, const void *hmp_dev, const void *off_dev, int
 }
 
 int og_plan_launch(og_handle *h, int32_t plan_id, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && plan_id >= 0 && plan_id < h->n_plans, "og_plan_launch: unknown plan %d", plan_id);
     const og_handle::Plan &p = h->plans[plan_id];
     OG_REQUIRE(!p.flip_test || p.tables_version == h->tables_version,
@@ -1449,6 +1467,7 @@ int og_decode_features_host(og_handle *h, const float *hmp_host, const float *of
                             int hgt, int w, int hmp_stride, int off_stride, int resize_mode,
                             int flip_test, const int32_t *kp_flip, const int32_t *limb_flip,
                             const int32_t *limb_reserve, int n_reserve, void *stream) {
+    StagedFramesOfCall frames_of_call{h};
     OG_REQUIRE(h && (n == 0 || (hmp_host && off_host)), "og_decode_features_host: null pointer");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     OG_TRY(check_feature_args(h, n, hgt, w, hmp_stride, off_stride, resize_mode, flip_test, kp_flip,

@@ -5,6 +5,7 @@ import collections
 import logging
 import re
 
+import numpy as np
 import torch
 
 from .. import config
@@ -124,7 +125,13 @@ class PostProcess(torch.nn.Module):
         tables = self._flip_tables if flip_test else None
         poses = eng.decode_features(hmps, offs, self.hmp_stride, self.off_stride, self.inter_mode, tables,
                                     frames=results.frames_of(metas))
-        return (poses,) + results.result_arrays(eng.last_result_rows, len(self.keypoints))
+        rows = eng.last_result_rows
+        if rows is None and not poses:
+            # an empty batch runs no kernel, so nothing wrote rows; the reference's loops make none
+            c = len(self.keypoints)
+            rows = (np.zeros((0, 3 * c), np.float32), np.zeros((0,), np.float64), np.zeros((0,), np.int32),
+                    np.zeros((0,), np.int32))
+        return (poses,) + results.result_arrays(rows, len(self.keypoints))
 
     # ---- pipelined form of generate_poses ------------------------------------------------------
     # The reference call is synchronous: the host waits for every batch.  A decode of a few images

@@ -378,9 +378,8 @@ class DecoderEngine(object):
         either CUDA tensors or CPU tensors (pinned memory gives asynchronous copies).
         ``flip_tables`` = (kp_flips, limb_flips, limb_reserve) enables flip fusion; the
         inputs then hold the originals followed by the W-flipped copies.  ``frames``: see
-        ``stage_frames``."""
-        if frames is not None:
-            self.stage_frames(frames)
+        ``stage_frames``; they are staged right before the library call, after every check here,
+        so that a call refused on the way does not leave them to the next one."""
         on_host = not hmp.is_cuda
         flip = flip_tables is not None
         if not on_host:
@@ -394,6 +393,8 @@ class DecoderEngine(object):
             if hit is not None and (not flip or hit[3] is flip_tables):
                 fn, args, n, _ = hit
                 stream = ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+                if frames is not None:
+                    self.stage_frames(frames)
                 if torch.cuda.current_device() == self.device.index:
                     st = fn(*args, stream)
                 else:
@@ -445,6 +446,8 @@ class DecoderEngine(object):
             call = (self._h, _ptr(hmp), _ptr(off), n, h, w, int(hmp_stride), int(off_stride),
                     mode, 1 if flip else 0) + tuple(args)
         with torch.cuda.device(self.device):
+            if frames is not None:
+                self.stage_frames(frames)
             _lib.check(fn(*call, _stream_ptr(self.device)))
         if not on_host and hmp is src_hmp and off is src_off:
             # the library was handed the caller's own buffers: the conversion can be reused
